@@ -23,10 +23,13 @@ the kernels) are compared with the oracle's sums all-reduced over torch.distribu
 `cpu_baseline` / `--impl reference`: the reference algorithm's CPU restatement (oracle/, OpenMP, fp64:
 one full pass per Brent evaluation as RDDLossFunction does) on the host cores, bounded sample.
 The reference itself is Scala/Spark and cannot run here (no JVM): kind = "port".
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed round returned (see dump_outputs) as
+DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -87,6 +90,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", "-i", str(self.gpu), f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                  "-lms", "200"], stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)  # nvidia-smi -lms never exits by itself: not even when bench.py fails
         except Exception:
             self.proc = None
 
@@ -250,6 +254,25 @@ def parity_check(ctx, n, lr, tol, max_iter, world, rank, dist, label):
             "r_max_rel_err": r_err, "tolerance": 1e-5, "seconds": time.perf_counter() - t_start}
 
 
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_ROWS = 1 << 21  # sampled rows: F and r in fp32 + the row indices in fp64 = 32 MB
+
+
+def dump_outputs(out_dir, ctx, n, alpha, loss_sum, n_eval):
+    """What a caller of the timed round receives after the last timed step: the line-search minimiser alpha, the train
+    loss sum and the number of Brent evaluations, and the round's per-row outputs — the updated predictions F and the
+    next pseudo-residuals r — over every row, or over a fixed seeded sample of DUMP_ROWS rows (`row_index`) when
+    there are more."""
+    from spark_ensemble_b200 import _native as N
+    idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    out = {"alpha": np.array([alpha]), "loss_sum": np.array([loss_sum]), "brent_evals": np.array([float(n_eval)]),
+           "row_index": idx.astype(np.float64),
+           "F": ctx.download(N.SLOT_F)[:n][idx], "r": ctx.download(N.SLOT_R)[:n][idx]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -266,7 +289,11 @@ def main():
                     help="GLOBAL rows of the strong-scaling measurement (split over the ranks); 0 disables")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle self-check after the timed regions")
     ap.add_argument("--no-extras", action="store_true", help="skip the tree / async / config-3 extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed round's outputs (rank 0) as DIR/<name>.npy, at most 32 MB")
     args = ap.parse_args()
+    if args.impl == "ours" and args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -352,8 +379,7 @@ def main():
 
     def step():
         # Brent line search + fused update/residual/loss: one call through the C ABI (se_gbm_round)
-        alpha, loss_sum, _ = ctx.gbm_round(lr, True, tol, max_iter, residual=True)
-        return alpha, loss_sum
+        return ctx.gbm_round(lr, True, tol, max_iter, residual=True)
 
     for _ in range(args.warmup):
         step()
@@ -365,7 +391,7 @@ def main():
     ctx.timer_start()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        last = step()
     ms_dev = ctx.timer_stop()
     ctx.sync()
     ms_wall = 1e3 * (time.perf_counter() - t0)
@@ -379,6 +405,8 @@ def main():
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, n, *last)
 
     # ---------------- e2e: host buffers through the host-side mirror's round body
     h_host, hp = _pinned_array(n)

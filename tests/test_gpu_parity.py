@@ -476,6 +476,41 @@ def test_multi_gpu_sharded_parity():
         assert f"p2p_allreduce={p2p == '1'}" in out.stdout
 
 
+def test_bench_dump_outputs_repeat(tmp_path):
+    """`bench.py --dump-outputs`: the last timed round's outputs over a seeded row sample, fp32 / fp64, within the
+    64 MB budget, and the same from one run to the next (the inputs are seeded)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, steps = 3_000_001, 2
+    dumps = []
+    for run in range(2):
+        d = tmp_path / f"run{run}"
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", "3",
+                              "--rows", str(n), "--no-features", "--no-extras", "--no-parity", "--strong-rows", "0",
+                              "--cpu-rows", "20000", "--dump-outputs", str(d)], capture_output=True, text=True,
+                             timeout=600)
+        assert out.returncode == 0, out.stderr[-4000:]
+        res = json.loads(out.stdout.strip().splitlines()[-1])
+        assert res["steps"] == steps and res["value"] > 0
+        files = sorted(os.listdir(d))
+        assert files == sorted(f"{k}.npy" for k in ("alpha", "loss_sum", "brent_evals", "row_index", "F", "r"))
+        assert sum(os.path.getsize(d / f) for f in files) <= 64 << 20
+        dumps.append({f[:-4]: np.load(d / f) for f in files})
+    a, b = dumps
+    for k, v in a.items():
+        assert v.dtype in (np.float32, np.float64), k
+    idx = a["row_index"]
+    assert idx.size == 1 << 21 and np.all(np.diff(idx) > 0) and idx[-1] < n and np.all(idx == np.floor(idx))
+    assert a["F"].shape == a["r"].shape == idx.shape and np.all(np.isfinite(a["F"])) and np.all(np.isfinite(a["r"]))
+    assert a["alpha"][0] > 0 and a["loss_sum"][0] > 0 and a["brent_evals"][0] >= 1
+    np.testing.assert_array_equal(a["row_index"], b["row_index"])
+    for k in ("alpha", "loss_sum", "F", "r"):
+        np.testing.assert_allclose(a[k], b[k], rtol=RTOL, atol=RTOL * float(np.abs(a[k]).max()), err_msg=k)
+
+
 @pytest.mark.parametrize("K", [9, 26, 32, 33, 64, 65, 200, 1000])
 @pytest.mark.parametrize("n", [1, 127, 129, 255, 256, 257, 40961])
 def test_logloss_wide_k_tiled_kernels(ctx, oracle, rng, K, n):
