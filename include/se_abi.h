@@ -330,6 +330,27 @@ SE_API int se_tree_predict_multi(se_ctx* ctx, int which, int n_nodes, const int3
 SE_API int se_forest_predict(se_ctx* ctx, int which, int n_trees, const int32_t* offsets, const int32_t* feature,
                              const float* threshold, const int32_t* left, const int32_t* right, const float* value,
                              const double* weights, double init, int out_slot, int out_row);
+/* A classifier ensemble of trees in ONE pass over the uint8 rank matrix of X (which = 0) or VX (which = 1), with no
+ * [M][K][n] member outputs.  Writes SE_SLOT_RAW [C][n], SE_SLOT_PROB [C][n] and SE_SLOT_LABEL [n] exactly as
+ * se_agg_configure(kind, M, num_classes, dim, loss, n) + se_agg_run(weights, init) would from the members' outputs.
+ * It allocates those three slots itself (n = columns of the feature slot) and never allocates SE_SLOT_P.
+ * Trees are concatenated as in se_forest_predict (offsets, tree-local children, GLOBAL columns).  Per kind:
+ *   SE_AGG_GBM_CLASSIFIER    M·dim trees, tree t = models(t / dim)(t % dim); leaf = regression value (leaf_width 1);
+ *                            weights [M][dim] (required), init [dim] or NULL (zeros)
+ *   SE_AGG_BAGGING_SOFT      M trees; leaf = class probabilities (leaf_width K); weights, init ignored
+ *   SE_AGG_BOOSTING_REAL     M trees; leaf = class probabilities (leaf_width K), summed as log(max(p, 2^-52)) formed
+ *                            once per leaf in fp64; weights, init ignored
+ *   SE_AGG_BAGGING_HARD      M trees; leaf = predicted label (leaf_width 1, K <= 65536); weights, init ignored
+ *   SE_AGG_BOOSTING_DISCRETE M trees; leaf = predicted label (leaf_width 1, K <= 65536); weights [M] (required)
+ * `leaf` is [total nodes][leaf_width] (internal nodes' entries are ignored).  A label leaf that is not an integer in
+ * [0, K), another kind, a leaf_width that does not match the kind, a node array that is not a tree or a column outside X
+ * fail with SE_ERR_ARG; a column that needs more than 255 thresholds (or no feature slot) with SE_ERR_STATE — evaluate
+ * the members with se_tree_predict* + se_agg_run then.  The class sums accumulate in fp64 in model order inside a chunk
+ * of trees and in RAW (fp32) between chunks; option last_forest_chunks reports the chunk count. */
+SE_API int se_forest_classify(se_ctx* ctx, int which, int kind, int num_classes, int dim, int loss,
+                              int n_trees, const int32_t* offsets, const int32_t* feature, const float* threshold,
+                              const int32_t* left, const int32_t* right, const float* leaf, int leaf_width,
+                              const double* weights, const double* init);
 /* linear model: out = intercept + Σ_j coef[j]·X[subspace[j]] */
 SE_API int se_linear_predict(se_ctx* ctx, int which, int n_coef, const float* coef, float intercept,
                       const int32_t* subspace, int out_slot, int out_row);

@@ -214,8 +214,8 @@ class GBMRegressorNative(override val uid: String) extends GBMRegressor(uid) {
 }
 
 /** Pre-order flattening of a Spark regression tree into the arrays se_tree_predict takes (continuous splits only). */
-private[regression] case class FlatTree(feature: Array[Int], threshold: Array[Float], left: Array[Int], right: Array[Int], value: Array[Float])
-private[regression] object FlatTree {
+private[ml] case class FlatTree(feature: Array[Int], threshold: Array[Float], left: Array[Int], right: Array[Int], value: Array[Float])
+private[ml] object FlatTree {
   import org.apache.spark.ml.tree.{ContinuousSplit, InternalNode, LeafNode, Node}
   def apply(model: DecisionTreeRegressionModel): FlatTree = {
     val f = scala.collection.mutable.ArrayBuffer[Int](); val t = scala.collection.mutable.ArrayBuffer[Float]()

@@ -16,7 +16,8 @@ from .ensemble import DataFrame, fit_dummy_classifier, java_string_hash, subspac
 from .gbm_engine import GBMEngine
 from .params import (Param, Params, ParamValidators, boosting_params, gbm_params, random_uid,
                      shared_classifier_params, shared_predictor_params, subbag_params)
-from .regression import _extract_instances, _split_validation, bag_counts
+from .regression import (_extract_instances, _forest_transform, _member_trees, _pforest, _split_validation,
+                         bag_counts)
 
 _CLS_LOSSES = ("logloss", "exponential", "bernoulli")  # GBMClassifier.scala:102-103
 _CLS_INIT = ("uniform", "prior")                        # :104-106
@@ -68,6 +69,18 @@ class _ClassifierModelBase(Params):
         label = ctx.download(N.SLOT_LABEL).astype(np.float64)
         C = self._out_classes
         return raw.reshape(C, -1).T, prob.reshape(C, -1).T, label
+
+    def _forest(self, X, trees, kind, subspaces=None, dim=1, loss=0, weights=None, init=None):
+        """Param forestTransform: the members' trees in one pass over X on the device (se_forest_classify).  None when
+        it is off, a member is not a tree, or the rank matrix cannot hold the forest: the member route runs then."""
+        if not self("forestTransform") or trees is None:
+            return None
+
+        def run(ctx):
+            ctx.forest_classify(trees, kind, self.numClasses, dim=dim, loss=loss, weights=weights, init=init,
+                                subspaces=subspaces)
+            return self._fetch(ctx)
+        return _forest_transform(self.device, X, run)
 
 
 # ================================================================================ GBMClassifier
@@ -194,9 +207,9 @@ _pcls = [
           lambda v: [int(d) for d in v]),
 ]
 _GBM_CLS_DEFAULTS = {**_d, **_dc, **_ds, **_db, **_dg, "loss": "logloss", "initStrategy": "prior",
-                     "residentFeatures": False, "lineSearch": "brent", "devices": [],
+                     "residentFeatures": False, "lineSearch": "brent", "devices": [], "forestTransform": False,
                      "seed": java_string_hash("org.apache.spark.ml.classification.GBMClassifier")}
-GBMClassifier._declare(_p + _pc + _ps + _pb + _pg + _pcls, _GBM_CLS_DEFAULTS)
+GBMClassifier._declare(_p + _pc + _ps + _pb + _pg + _pcls + _pforest, _GBM_CLS_DEFAULTS)
 
 
 class GBMClassificationModel(_ClassifierModelBase):
@@ -216,6 +229,12 @@ class GBMClassificationModel(_ClassifierModelBase):
 
     def _raw_prob_label(self, X):
         n, M, dim = X.shape[0], self.numModels, self.dim
+        if self("forestTransform"):  # tree t = models(t // dim)(t % dim)
+            trees = _member_trees([m for ms in self.models for m in ms])
+            res = self._forest(X, trees, N.AGG_GBM_CLASSIFIER, [s for s in self.subspaces for _ in range(dim)], dim,
+                               self("loss").lower(), np.stack(self.weights) if M else None, self.init)
+            if res is not None:
+                return res
         P = np.zeros((max(M, 1), dim, n), dtype=np.float32)
         for i in range(M):
             Xs = X[:, self.subspaces[i]]
@@ -229,7 +248,7 @@ class GBMClassificationModel(_ClassifierModelBase):
             return self._fetch(ctx)
 
 
-GBMClassificationModel._declare(_p + _pc + _ps + _pb + _pg + _pcls, _GBM_CLS_DEFAULTS)
+GBMClassificationModel._declare(_p + _pc + _ps + _pb + _pg + _pcls + _pforest, _GBM_CLS_DEFAULTS)
 
 
 # ================================================================================ BoostingClassifier
@@ -308,9 +327,9 @@ class BoostingClassifier(Params):
 _pboost = [Param("algorithm", "algorithm, (case-insensitive). Supported options: discrete,real",
                  lambda v: v.lower() in ("discrete", "real"), str),
            Param("residentFeatures", "evaluate base models on device over the HBM-resident feature matrix", convert=bool)]
-_BOOST_DEFAULTS = {**_d, **_dc, **_db, "algorithm": "discrete", "residentFeatures": False,
+_BOOST_DEFAULTS = {**_d, **_dc, **_db, "algorithm": "discrete", "residentFeatures": False, "forestTransform": False,
                    "seed": java_string_hash("org.apache.spark.ml.classification.BoostingClassifier")}
-BoostingClassifier._declare(_p + _pc + _pb + _pboost + [Param("seed", "random seed", convert=int)], _BOOST_DEFAULTS)
+BoostingClassifier._declare(_p + _pc + _pb + _pboost + _pforest + [Param("seed", "random seed", convert=int)], _BOOST_DEFAULTS)
 
 
 class BoostingClassificationModel(_ClassifierModelBase):
@@ -330,6 +349,11 @@ class BoostingClassificationModel(_ClassifierModelBase):
     def _raw_prob_label(self, X):
         n, M, K = X.shape[0], self.numModels, self.numClasses
         real = self("algorithm").lower() == "real"
+        res = self._forest(X, _member_trees(self.models) if self("forestTransform") else None,
+                           N.AGG_BOOSTING_REAL if real else N.AGG_BOOSTING_DISCRETE,
+                           weights=None if real else self.weights)
+        if res is not None:
+            return res
         with Context(self.device) as ctx:
             if real:
                 P = np.zeros((max(M, 1), K, n), dtype=np.float32)
@@ -350,7 +374,7 @@ class BoostingClassificationModel(_ClassifierModelBase):
             return self._fetch(ctx)
 
 
-BoostingClassificationModel._declare(_p + _pc + _pb + _pboost + [Param("seed", "random seed", convert=int)], _BOOST_DEFAULTS)
+BoostingClassificationModel._declare(_p + _pc + _pb + _pboost + _pforest + [Param("seed", "random seed", convert=int)], _BOOST_DEFAULTS)
 
 
 # ================================================================================ BaggingClassifier
@@ -385,8 +409,9 @@ _pbagc = [Param("numBaseLearners", "number of base learners", ParamValidators.gt
                 lambda v: v.lower() in ("soft", "hard"), str),
           Param("parallelism", "threads", ParamValidators.gtEq(1), int)]
 _BAG_CLS_DEFAULTS = {**_d, **_dc, **_ds, "numBaseLearners": 10, "votingStrategy": "hard", "parallelism": 1,
+                     "forestTransform": False,
                      "seed": java_string_hash("org.apache.spark.ml.classification.BaggingClassifier")}
-BaggingClassifier._declare(_p + _pc + _ps + _pbagc, _BAG_CLS_DEFAULTS)
+BaggingClassifier._declare(_p + _pc + _ps + _pbagc + _pforest, _BAG_CLS_DEFAULTS)
 
 
 class BaggingClassificationModel(_ClassifierModelBase):
@@ -404,6 +429,10 @@ class BaggingClassificationModel(_ClassifierModelBase):
     def _raw_prob_label(self, X):
         n, M, K = X.shape[0], self.numModels, self.numClasses
         soft = self("votingStrategy").lower() == "soft"
+        res = self._forest(X, _member_trees(self.models) if self("forestTransform") else None,
+                           N.AGG_BAGGING_SOFT if soft else N.AGG_BAGGING_HARD, self.subspaces)
+        if res is not None:
+            return res
         with Context(self.device) as ctx:
             if soft:
                 P = np.zeros((M, K, n), dtype=np.float32)
@@ -420,4 +449,4 @@ class BaggingClassificationModel(_ClassifierModelBase):
             return self._fetch(ctx)
 
 
-BaggingClassificationModel._declare(_p + _pc + _ps + _pbagc, _BAG_CLS_DEFAULTS)
+BaggingClassificationModel._declare(_p + _pc + _ps + _pbagc + _pforest, _BAG_CLS_DEFAULTS)

@@ -12,6 +12,28 @@ import numpy as np
 from . import _native as N
 
 
+def _flatten_trees(trees, subspaces, leaf_key):
+    """Concatenated node arrays of a forest (offsets, feature, threshold, left, right, leaf) as se_forest_predict /
+    se_forest_classify take them: tree-local children, features mapped through each tree's subspace to GLOBAL columns,
+    tree[leaf_key] flattened per node ([n_nodes] or [n_nodes, width])."""
+    offs = np.zeros(len(trees) + 1, dtype=np.int32)
+    f, t, l, r, v = [], [], [], [], []
+    for i, tr in enumerate(trees):
+        fi = np.asarray(tr["feature"], dtype=np.int32)
+        if subspaces is not None and subspaces[i] is not None:
+            sub = np.asarray(subspaces[i], dtype=np.int32)
+            if np.any(fi >= sub.size):
+                raise ValueError(f"tree {i}: feature index outside its subspace")
+            fi = np.where(fi >= 0, sub[np.maximum(fi, 0)], fi).astype(np.int32)
+        f.append(fi)
+        t.append(np.asarray(tr["threshold"], dtype=np.float32))
+        l.append(np.asarray(tr["left"], dtype=np.int32))
+        r.append(np.asarray(tr["right"], dtype=np.int32))
+        v.append(np.asarray(tr[leaf_key], dtype=np.float32).reshape(-1))
+        offs[i + 1] = offs[i] + fi.size
+    return (offs,) + tuple(np.ascontiguousarray(np.concatenate(a)) for a in (f, t, l, r, v))
+
+
 class Context:
     def __init__(self, device: int = 0):
         self._lib = N.load()
@@ -379,28 +401,33 @@ class Context:
         """out = init + sum_t weights[t] * tree_t(x) for a list of regression trees (dicts as in tree_predict) in one
         pass over the resident feature matrix (se_forest_predict: GBMRegressionModel.predict,
         regression/GBMRegressor.scala:531-539).  `subspaces[t]` maps tree t's feature indices to columns of X."""
-        offs = np.zeros(len(trees) + 1, dtype=np.int32)
-        f, t, l, r, v = [], [], [], [], []
-        for i, tr in enumerate(trees):
-            fi = np.asarray(tr["feature"], dtype=np.int32)
-            if subspaces is not None and subspaces[i] is not None:
-                sub = np.asarray(subspaces[i], dtype=np.int32)
-                if np.any(fi >= sub.size):
-                    raise ValueError(f"tree {i}: feature index outside its subspace")
-                fi = np.where(fi >= 0, sub[np.maximum(fi, 0)], fi).astype(np.int32)
-            f.append(fi)
-            t.append(np.asarray(tr["threshold"], dtype=np.float32))
-            l.append(np.asarray(tr["left"], dtype=np.int32))
-            r.append(np.asarray(tr["right"], dtype=np.int32))
-            v.append(np.asarray(tr["value"], dtype=np.float32))
-            offs[i + 1] = offs[i] + fi.size
-        f, t, l, r, v = (np.ascontiguousarray(np.concatenate(a)) for a in (f, t, l, r, v))
+        offs, f, t, l, r, v = _flatten_trees(trees, subspaces, "value")
         w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
         if w is not None and w.size != len(trees):
             raise ValueError("one weight per tree")
         self._ck(self._lib.se_forest_predict(self._h, int(validation), len(trees), N.iptr(offs), N.iptr(f), N.fptr(t),
                                              N.iptr(l), N.iptr(r), N.fptr(v), None if w is None else N.dptr(w),
                                              float(init), out_slot, out_row))
+
+    def forest_classify(self, trees, kind: int, num_classes: int, dim: int = 1, loss=0, weights=None, init=None,
+                        validation: bool = False, subspaces=None):
+        """RAW, PROB and LABEL of a classifier ensemble of trees in one pass over the resident feature matrix
+        (se_forest_classify): what agg_configure + agg_run would give from the members' outputs, without them.
+        Leaves: tree["values"] ([n_nodes, K] class probabilities) for AGG_BAGGING_SOFT / AGG_BOOSTING_REAL,
+        tree["value"] (regression value or predicted label) for the others.  GBM: tree t = models(t // dim)(t % dim),
+        weights [M][dim], init [dim]; SAMME: weights [M].  `subspaces[t]` maps tree t's features to columns of X."""
+        vector = kind in (N.AGG_BAGGING_SOFT, N.AGG_BOOSTING_REAL)
+        offs, f, t, l, r, v = _flatten_trees(trees, subspaces, "values" if vector else "value")
+        width = v.size // max(int(offs[-1]), 1)
+        lid = N.LOSS[loss] if isinstance(loss, str) else int(loss)
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64).reshape(-1)
+        if w is not None and w.size != len(trees):
+            raise ValueError("one weight per tree")
+        i = None if init is None else np.ascontiguousarray(np.atleast_1d(init), dtype=np.float64)
+        self._ck(self._lib.se_forest_classify(self._h, int(validation), int(kind), int(num_classes), int(dim), lid,
+                                              len(trees), N.iptr(offs), N.iptr(f), N.fptr(t), N.iptr(l), N.iptr(r),
+                                              N.fptr(v), int(width), None if w is None else N.dptr(w),
+                                              None if i is None else N.dptr(i)))
 
     def linear_predict(self, coef, intercept: float, out_slot: int, out_row: int = 0,
                        validation: bool = False, subspace=None):

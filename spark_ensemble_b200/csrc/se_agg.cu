@@ -1108,4 +1108,15 @@ cudaError_t launch_agg(const AggArgs& a, int ctas_per_sm, int sms, cudaStream_t 
   return cudaGetLastError();
 }
 
+cudaError_t launch_agg_finalize(int kind, int C, int K, int dim, int loss, int M, double sum_a, int64_t n, int64_t ld,
+                                float* raw, float* prob, float* label, int sms, cudaStream_t st) {
+  FinArgs f{};
+  f.kind = kind; f.C = C; f.K = K; f.dim = dim; f.loss = loss; f.M = M;
+  f.sum_a = sum_a;
+  f.n = n; f.ld = ld; f.raw = raw; f.prob = prob; f.label = label;
+  f.inv_km1 = 1.0 / (double)((K > 1 ? K : 2) - 1);
+  agg_finalize_kernel<<<grid_rows(n, kBlock, 8, sms), kBlock, 0, st>>>(f);
+  return cudaGetLastError();
+}
+
 }  // namespace se

@@ -245,8 +245,10 @@ struct se_ctx {
   // binned (uint8) copies of X / VX for the tree walk
   BinState bins[2];
   int tree_bins = 1;                  // 0: always walk the fp32 matrix
-  unsigned char* d_forest = nullptr;  // packed chunk of trees for se_forest_predict
+  unsigned char* d_forest = nullptr;  // packed chunk of trees for se_forest_predict / se_forest_classify
   size_t forest_cap = 0;
+  float* d_forest_leaves = nullptr;   // leaf table of se_forest_classify (every tree's leaves, one or K floats each)
+  size_t forest_leaves_cap = 0;
   int last_forest_chunks = 0;
   int wm_fast = 1;                    // weighted median (M <= 64, weights >= 0): keys-only sort + margin check, exact kernel for the rest
   int64_t wm_list_cap = 0;            // deferred-row list capacity (0: n / 4)
@@ -755,6 +757,7 @@ int se_ctx_destroy(se_ctx* ctx) {
   free_bins(ctx->bins[1]);
   if (ctx->d_wm) cudaFree(ctx->d_wm);
   if (ctx->d_forest) cudaFree(ctx->d_forest);
+  if (ctx->d_forest_leaves) cudaFree(ctx->d_forest_leaves);
   if (ctx->big.d_coef) cudaFree(ctx->big.d_coef);
   if (ctx->big.h_coef) cudaFreeHost(ctx->big.h_coef);
   if (ctx->big.d_partials) cudaFree(ctx->big.d_partials);
@@ -2683,6 +2686,132 @@ int se_tree_predict_multi(se_ctx* ctx, int which, int n_nodes, const int32_t* fe
                            out_slot, 0);
 }
 
+// ---- tree ensembles in one pass over the rank matrix (se_forest_predict, se_forest_classify) ----------------------
+namespace {
+// Every member must be a tree rooted at its first node, with tree-local child indices and GLOBAL column indices of X
+// (the device walk follows child links until it meets a leaf: a node reached twice could make it spin forever).
+int forest_validate(se_ctx* ctx, const SlotBuf& X, int n_trees, const int32_t* offsets, const int32_t* feature,
+                    const int32_t* left, const int32_t* right) {
+  SE_REQUIRE(ctx, n_trees >= 1 && n_trees <= (1 << 20), SE_ERR_ARG, "bad tree count %d", n_trees);
+  SE_REQUIRE(ctx, offsets[0] == 0, SE_ERR_ARG, "offsets[0] must be 0");
+  const int64_t total = offsets[n_trees];
+  SE_REQUIRE(ctx, total >= n_trees && total <= (1 << 26), SE_ERR_ARG, "bad node count %lld", (long long)total);
+  std::vector<char> seen;
+  std::vector<int32_t> stack;
+  for (int t = 0; t < n_trees; ++t) {
+    const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
+    SE_REQUIRE(ctx, nn >= 1 && nn <= 65535, SE_ERR_ARG, "tree %d: %d nodes (1..65535 supported)", t, nn);
+    for (int i = 0; i < nn; ++i) {
+      if (feature[b + i] < 0) continue;
+      SE_REQUIRE(ctx, feature[b + i] < X.rows, SE_ERR_ARG, "tree %d node %d: column %d outside X with %lld columns", t, i,
+                 feature[b + i], (long long)X.rows);
+      SE_REQUIRE(ctx, left[b + i] >= 0 && left[b + i] < nn && right[b + i] >= 0 && right[b + i] < nn, SE_ERR_ARG,
+                 "tree %d node %d: bad child", t, i);
+    }
+    seen.assign((size_t)nn, 0);
+    stack.clear();
+    stack.push_back(0);
+    seen[0] = 1;
+    while (!stack.empty()) {
+      const int32_t i = stack.back();
+      stack.pop_back();
+      if (feature[b + i] < 0) continue;
+      for (const int32_t c : {left[b + i], right[b + i]}) {
+        SE_REQUIRE(ctx, !seen[c], SE_ERR_ARG, "tree %d: node %d is reached twice: not a tree", t, c);
+        seen[c] = 1;
+        stack.push_back(c);
+      }
+    }
+  }
+  return SE_OK;
+}
+
+// The forest kernels compare ranks, not features: every threshold of the forest must have a rank in the uint8 matrix.
+int forest_ranks(se_ctx* ctx, int which, const SlotBuf& X, int64_t total, const int32_t* feature, const float* threshold) {
+  const int rc = bins_prepare(ctx, which, X, (int)total, feature, threshold);
+  if (rc < 0) return rc;
+  SE_REQUIRE(ctx, rc == 1, SE_ERR_STATE,
+             "the forest kernel needs the uint8 rank matrix (tree_bins on, <= 255 distinct thresholds per column, no NaN "
+             "threshold): evaluate the members with se_tree_predict + se_agg_run instead");
+  return SE_OK;
+}
+
+size_t pad_to(size_t v, size_t to) { return (v + to - 1) / to * to; }
+
+// Grows the chunk of trees order[p0..p1) (order == nullptr: identity) tree by tree while bytes(trees, columns, nodes),
+// the kernel's shared memory, fits the budget; a member that does not fit the four-CTAs-per-SM budget alone gets two,
+// then one CTA per SM.  On return `used` lists the chunk's global columns and local[] maps them to their position.
+// Returns p1 (== p0: even one tree does not fit).
+int forest_chunk(const int32_t* order, int p0, int n_trees, const int32_t* offsets, const int32_t* feature,
+                 std::vector<int32_t>& local, std::vector<int32_t>& used, size_t& nodes,
+                 size_t (*bytes)(size_t T, size_t C, size_t Nn)) {
+  int p1 = p0;
+  for (const size_t budget : {(size_t)kForestSmemBudget, (size_t)(100 * 1024), (size_t)(216 * 1024)}) {
+    for (int32_t c : used) local[c] = -1;
+    used.clear();
+    nodes = 0;
+    for (p1 = p0; p1 < n_trees; ++p1) {
+      const int t = order ? order[p1] : p1;
+      const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
+      std::vector<int32_t> added;
+      for (int i = 0; i < nn; ++i) {
+        const int32_t c = feature[b + i];
+        if (c >= 0 && local[c] < 0) { local[c] = (int32_t)(used.size() + added.size()); added.push_back(c); }
+      }
+      const size_t T = (size_t)(p1 - p0 + 1), C = used.size() + added.size(), Nn = nodes + (size_t)nn;
+      if (bytes(T, C, Nn) > budget || C > 65535) {
+        for (int32_t c : added) local[c] = -1;
+        break;
+      }
+      used.insert(used.end(), added.begin(), added.end());
+      nodes = Nn;
+    }
+    if (p1 > p0) break;
+  }
+  return p1;
+}
+
+// Packed nodes of one tree: x = local column | rank threshold << 16 | leaf << 31; y = left | right << 16 (tree-local)
+// for an internal node, the leaf's ordinal among the tree's leaves (node order) for a leaf.  Returns the leaf count.
+int forest_pack_tree(const BinState& B, const std::vector<int32_t>& local, int32_t b, int32_t nn, const int32_t* feature,
+                     const float* threshold, const int32_t* left, const int32_t* right, uint2* out) {
+  int leaves = 0;
+  for (int i = 0; i < nn; ++i) {
+    const int32_t c = feature[b + i];
+    if (c < 0) { out[i] = make_uint2(0x80000000u, (uint32_t)leaves++); continue; }
+    const std::vector<float>& E = B.edges[c];
+    const uint32_t j = (uint32_t)(std::lower_bound(E.begin(), E.end(), threshold[b + i]) - E.begin());  // x <= t_j <=> rank <= j
+    out[i] = make_uint2((uint32_t)local[c] | (j << 16), (uint32_t)left[b + i] | ((uint32_t)right[b + i] << 16));
+  }
+  return leaves;
+}
+
+// Copies a packed chunk into ctx->d_forest (grown on demand).
+int forest_upload_blob(se_ctx* ctx, const std::vector<unsigned char>& blob) {
+  if (ctx->forest_cap < blob.size()) {
+    if (ctx->d_forest) cudaFree(ctx->d_forest);
+    ctx->d_forest = nullptr; ctx->forest_cap = 0;
+    SE_CUDA(ctx, cudaMalloc(&ctx->d_forest, blob.size()));
+    ctx->forest_cap = blob.size();
+  }
+  // the previous chunk's kernel may still be reading d_forest
+  SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  SE_CUDA(ctx, cudaMemcpyAsync(ctx->d_forest, blob.data(), blob.size(), cudaMemcpyHostToDevice, ctx->stream));
+  SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // blob is pageable host memory reused by the next chunk
+  return SE_OK;
+}
+
+size_t forest_predict_bytes(size_t T, size_t C, size_t Nn) {
+  return pad_to(8 * T + 8 * C + 8 * Nn + pad_to(4 * (T + 1), 8) + pad_to(4 * Nn, 16), 16) + C * kForestTile;
+}
+
+// se_forest_classify's blob (ForestClassArgs) with at most T classes in a chunk, the ranks and the parked leaves
+size_t forest_classify_bytes(size_t T, size_t C, size_t Nn) {
+  return pad_to(8 * T + 8 * T + 8 * C + 8 * Nn + 4 * (T + 1) + 4 * T + 4 * (T + 1), 16) + pad_to(C * kForestTile, 16) +
+         T * kForestTile * sizeof(uint16_t);
+}
+}  // namespace
+
 // Σ_t weights[t] · tree_t(x) + init for every row in one pass over the rank matrix per chunk of trees
 // (GBMRegressionModel.predict, regression/GBMRegressor.scala:531-539; BaggingRegressionModel.predict,
 // regression/BaggingRegressor.scala:221-228 with weights 1 / M).
@@ -2690,94 +2819,31 @@ int se_forest_predict(se_ctx* ctx, int which, int n_trees, const int32_t* offset
                       const float* threshold, const int32_t* left, const int32_t* right, const float* value,
                       const double* weights, double init, int out_slot, int out_row) {
   if (!ctx || !offsets || !feature || !threshold || !left || !right || !value) return fail(ctx, SE_ERR_ARG, "null argument");
-  SE_REQUIRE(ctx, n_trees >= 1 && n_trees <= (1 << 20), SE_ERR_ARG, "bad tree count %d", n_trees);
   SE_REQUIRE(ctx, out_slot >= 0 && out_slot < SE_NUM_SLOTS, SE_ERR_ARG, "bad out slot");
   const SlotBuf& X = ctx->slot[which ? SE_SLOT_VX : SE_SLOT_X];
   const SlotBuf& O = ctx->slot[out_slot];
   SE_REQUIRE(ctx, X.d, SE_ERR_STATE, "feature matrix slot not allocated");
   SE_REQUIRE(ctx, O.d && O.cols == X.cols && out_row >= 0 && out_row < O.rows, SE_ERR_STATE, "output slot shape mismatch");
-  SE_REQUIRE(ctx, offsets[0] == 0, SE_ERR_ARG, "offsets[0] must be 0");
+  SE_TRY(forest_validate(ctx, X, n_trees, offsets, feature, left, right));
   const int64_t total = offsets[n_trees];
-  SE_REQUIRE(ctx, total >= n_trees && total <= (1 << 26), SE_ERR_ARG, "bad node count %lld", (long long)total);
-  // every member must be a tree rooted at its first node, with tree-local child indices and GLOBAL column indices
-  {
-    std::vector<char> seen;
-    std::vector<int32_t> stack;
-    for (int t = 0; t < n_trees; ++t) {
-      const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
-      SE_REQUIRE(ctx, nn >= 1 && nn <= 65535, SE_ERR_ARG, "tree %d: %d nodes (1..65535 supported)", t, nn);
-      for (int i = 0; i < nn; ++i) {
-        if (feature[b + i] < 0) continue;
-        SE_REQUIRE(ctx, feature[b + i] < X.rows, SE_ERR_ARG, "tree %d node %d: column %d outside X with %lld columns", t, i,
-                   feature[b + i], (long long)X.rows);
-        SE_REQUIRE(ctx, left[b + i] >= 0 && left[b + i] < nn && right[b + i] >= 0 && right[b + i] < nn, SE_ERR_ARG,
-                   "tree %d node %d: bad child", t, i);
-      }
-      seen.assign((size_t)nn, 0);
-      stack.clear();
-      stack.push_back(0);
-      seen[0] = 1;
-      while (!stack.empty()) {
-        const int32_t i = stack.back();
-        stack.pop_back();
-        if (feature[b + i] < 0) continue;
-        for (const int32_t c : {left[b + i], right[b + i]}) {
-          SE_REQUIRE(ctx, !seen[c], SE_ERR_ARG, "tree %d: node %d is reached twice: not a tree", t, c);
-          seen[c] = 1;
-          stack.push_back(c);
-        }
-      }
-    }
-  }
   SE_TRY(begin(ctx));
   release_l2_persist(ctx);
   SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  {
-    const int rc = bins_prepare(ctx, which, X, (int)total, feature, threshold);
-    if (rc < 0) return rc;
-    SE_REQUIRE(ctx, rc == 1, SE_ERR_STATE,
-               "the forest kernel needs the uint8 rank matrix (tree_bins on, <= 255 distinct thresholds per column, no NaN "
-               "threshold): evaluate the members with se_tree_predict + se_agg_run instead");
-  }
+  SE_TRY(forest_ranks(ctx, which, X, total, feature, threshold));
   BinState& B = ctx->bins[which];
   if (out_slot == SE_SLOT_F || out_slot == SE_SLOT_R || out_slot == SE_SLOT_Y) ctx->gbm.r_current = false;
   ForestArgs a;
   a.X8 = B.d8; a.n = X.cols; a.ld8 = B.ld8;
   a.out = O.d + (int64_t)out_row * (O.rows > 1 ? O.ld : O.cols);
   a.init = init;
-  auto pad = [](size_t v, size_t to) { return (v + to - 1) / to * to; };
   std::vector<int32_t> local((size_t)X.rows, -1);  // global column -> local column of the current chunk
   std::vector<int32_t> used;
   std::vector<unsigned char> blob;
   int chunks = 0;
   int t0 = 0;
   while (t0 < n_trees) {
-    // grow the chunk tree by tree while columns x 256 ranks + packed trees fit the shared-memory budget
     size_t nodes = 0;
-    int t1 = t0;
-    // a member that does not fit the four-CTAs-per-SM budget alone gets two, then one CTA per SM
-    for (const size_t budget : {(size_t)kForestSmemBudget, (size_t)(100 * 1024), (size_t)(216 * 1024)}) {
-    for (int32_t c : used) local[c] = -1;
-    used.clear();
-    nodes = 0;
-    for (t1 = t0; t1 < n_trees; ++t1) {
-      const int32_t b = offsets[t1], nn = offsets[t1 + 1] - offsets[t1];
-      std::vector<int32_t> added;
-      for (int i = 0; i < nn; ++i) {
-        const int32_t c = feature[b + i];
-        if (c >= 0 && local[c] < 0) { local[c] = (int32_t)(used.size() + added.size()); added.push_back(c); }
-      }
-      const size_t T = (size_t)(t1 - t0 + 1), C = used.size() + added.size(), Nn = nodes + (size_t)nn;
-      const size_t bytes = pad(8 * T + 8 * C + 8 * Nn + pad(4 * (T + 1), 8) + pad(4 * Nn, 16), 16) + C * kForestTile;
-      if (bytes > budget || C > 65535) {
-        for (int32_t c : added) local[c] = -1;
-        break;
-      }
-      used.insert(used.end(), added.begin(), added.end());
-      nodes = Nn;
-    }
-    if (t1 > t0) break;
-    }
+    const int t1 = forest_chunk(nullptr, t0, n_trees, offsets, feature, local, used, nodes, forest_predict_bytes);
     SE_REQUIRE(ctx, t1 > t0, SE_ERR_ARG, "tree %d alone (%d nodes) does not fit the forest kernel's shared memory", t0,
                offsets[t0 + 1] - offsets[t0]);
     const size_t T = (size_t)(t1 - t0), C = used.size(), Nn = nodes;
@@ -2785,8 +2851,8 @@ int se_forest_predict(se_ctx* ctx, int which, int n_trees, const int32_t* offset
     a.off_coloff = (int)(8 * T);
     a.off_nodes = a.off_coloff + (int)(8 * C);
     a.off_treeoff = a.off_nodes + (int)(8 * Nn);
-    a.off_values = a.off_treeoff + (int)pad(4 * (T + 1), 8);
-    a.blob_bytes = (int)pad((size_t)a.off_values + 4 * Nn, 16);
+    a.off_values = a.off_treeoff + (int)pad_to(4 * (T + 1), 8);
+    a.blob_bytes = (int)pad_to((size_t)a.off_values + 4 * Nn, 16);
     a.off_ranks = a.blob_bytes;
     blob.assign((size_t)a.blob_bytes, 0);
     double* bw = reinterpret_cast<double*>(blob.data());
@@ -2800,33 +2866,159 @@ int se_forest_predict(se_ctx* ctx, int which, int n_trees, const int32_t* offset
       const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
       bw[t - t0] = weights ? weights[t] : 1.0;
       bto[t - t0] = (int32_t)at;
-      for (int i = 0; i < nn; ++i) {
-        const int32_t c = feature[b + i];
-        bv[at + i] = value[b + i];
-        if (c < 0) { bn[at + i] = make_uint2(0x80000000u, 0u); continue; }
-        const std::vector<float>& E = B.edges[c];
-        const uint32_t j = (uint32_t)(std::lower_bound(E.begin(), E.end(), threshold[b + i]) - E.begin());  // x <= t_j <=> rank <= j
-        bn[at + i] = make_uint2((uint32_t)local[c] | (j << 16), (uint32_t)left[b + i] | ((uint32_t)right[b + i] << 16));
-      }
+      forest_pack_tree(B, local, b, nn, feature, threshold, left, right, bn + at);
+      for (int i = 0; i < nn; ++i) bv[at + i] = value[b + i];
       at += (size_t)nn;
     }
     bto[T] = (int32_t)at;
-    if (ctx->forest_cap < (size_t)a.blob_bytes) {
-      if (ctx->d_forest) cudaFree(ctx->d_forest);
-      ctx->d_forest = nullptr; ctx->forest_cap = 0;
-      SE_CUDA(ctx, cudaMalloc(&ctx->d_forest, (size_t)a.blob_bytes));
-      ctx->forest_cap = (size_t)a.blob_bytes;
-    }
-    // the previous chunk's kernel may still be reading d_forest
-    SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    SE_CUDA(ctx, cudaMemcpyAsync(ctx->d_forest, blob.data(), (size_t)a.blob_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // blob is pageable host memory reused by the next chunk
+    SE_TRY(forest_upload_blob(ctx, blob));
     a.blob = ctx->d_forest;
     a.accumulate = chunks > 0 ? 1 : 0;
     SE_LAUNCH_T(ctx, SE_KF_TREE, launch_forest_predict(a, ctx->sms, ctx->stream));
     ++chunks;
     t0 = t1;
   }
+  ctx->last_forest_chunks = chunks;
+  ctx->last_tree_binned = 1;
+  return end(ctx);
+}
+
+// predictRaw / raw2probability / raw2prediction of a classifier ensemble of trees in one pass over the rank matrix per
+// chunk of trees: the stage-1 class sums se_agg_run forms from the members' outputs (GBMClassifier.scala:567-589,
+// BaggingClassifier.scala:260-283, BoostingClassifier.scala:348-382) go straight to RAW, then the aggregation's own
+// epilogue turns them into raw, probability and label.  No [M][K][n] member outputs exist at any point.
+int se_forest_classify(se_ctx* ctx, int which, int kind, int num_classes, int dim, int loss, int n_trees,
+                       const int32_t* offsets, const int32_t* feature, const float* threshold, const int32_t* left,
+                       const int32_t* right, const float* leaf, int leaf_width, const double* weights, const double* init) {
+  if (!ctx || !offsets || !feature || !threshold || !left || !right || !leaf) return fail(ctx, SE_ERR_ARG, "null argument");
+  const int K = num_classes;
+  SE_REQUIRE(ctx, kind >= SE_AGG_GBM_CLASSIFIER && kind <= SE_AGG_BOOSTING_DISCRETE, SE_ERR_ARG,
+             "kind %d is not a classifier aggregation", kind);
+  SE_REQUIRE(ctx, K >= 2, SE_ERR_ARG, "numClasses >= 2");
+  const bool gbm = kind == SE_AGG_GBM_CLASSIFIER;
+  const bool labels = kind == SE_AGG_BAGGING_HARD || kind == SE_AGG_BOOSTING_DISCRETE;
+  const int mode = gbm ? kForestScalarLeaves : labels ? kForestLabelLeaves : kForestVectorLeaves;
+  const int want_width = (mode == kForestVectorLeaves) ? K : 1;
+  SE_REQUIRE(ctx, leaf_width == want_width, SE_ERR_ARG, "kind %d takes leaves of width %d (got %d)", kind, want_width, leaf_width);
+  SE_REQUIRE(ctx, !gbm || (dim >= 1 && n_trees % dim == 0), SE_ERR_ARG, "GBM: %d trees are not rounds of dim %d", n_trees, dim);
+  SE_REQUIRE(ctx, !labels || K <= 65536, SE_ERR_ARG, "label leaves: at most 65536 classes (got %d)", K);
+  SE_REQUIRE(ctx, weights || !(gbm || kind == SE_AGG_BOOSTING_DISCRETE), SE_ERR_ARG, "weights required for this aggregation kind");
+  const SlotBuf& X = ctx->slot[which ? SE_SLOT_VX : SE_SLOT_X];
+  SE_REQUIRE(ctx, X.d, SE_ERR_STATE, "feature matrix slot not allocated");
+  SE_TRY(forest_validate(ctx, X, n_trees, offsets, feature, left, right));
+  const int64_t total = offsets[n_trees];
+  // a label leaf is a class index: checked here once per leaf instead of once per row on the device
+  if (labels)
+    for (int64_t i = 0; i < total; ++i) {
+      if (feature[i] >= 0) continue;
+      const float v = leaf[i];
+      SE_REQUIRE(ctx, v >= 0.f && v < (float)K && v == floorf(v), SE_ERR_ARG, "node %lld: leaf label %g is not a class in [0, %d)",
+                 (long long)i, (double)v, K);
+    }
+  const int S = gbm ? dim : K;                           // classes with a stage-1 sum
+  const int Cout = (gbm && dim == 1 && K == 2) ? 2 : S;  // rows of RAW / PROB (binary GBM: (-F, F))
+  const int M = gbm ? n_trees / dim : n_trees;
+  // leaf table: every tree's leaves in node order, one value (GBM, label) or K values (class probabilities) each;
+  // SAMME.R sums log(max(p, eps)) (BoostingClassifier.scala:352-354): formed here once per leaf, in fp64
+  std::vector<int32_t> lbase((size_t)n_trees);
+  std::vector<float> lv;
+  for (int t = 0; t < n_trees; ++t) {
+    lbase[t] = (int32_t)lv.size();
+    for (int32_t i = offsets[t]; i < offsets[t + 1]; ++i) {
+      if (feature[i] >= 0) continue;
+      for (int k = 0; k < want_width; ++k) {
+        const double p = leaf[(size_t)i * want_width + k];
+        lv.push_back(kind == SE_AGG_BOOSTING_REAL ? (float)log(fmax(p, 2.220446049250313e-16)) : (float)p);
+      }
+      SE_REQUIRE(ctx, lv.size() <= (size_t)INT32_MAX, SE_ERR_ARG, "leaf table of more than 2^31 values");
+    }
+  }
+  // GBM: tree t is models(t / dim)(t % dim) and adds to class t % dim only — order the trees class-major (rounds in model
+  // order inside a class), so a chunk covers a contiguous range of classes; the other kinds add to every class.
+  std::vector<int32_t> order((size_t)n_trees);
+  for (int p = 0; p < n_trees; ++p) order[p] = gbm ? (p % M) * dim + p / M : p;
+  double sum_a = 0.0;
+  if (kind == SE_AGG_BOOSTING_DISCRETE)
+    for (int t = 0; t < n_trees; ++t) sum_a += weights[t];
+  SE_TRY(begin(ctx));
+  release_l2_persist(ctx);
+  SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  SE_TRY(forest_ranks(ctx, which, X, total, feature, threshold));
+  BinState& B = ctx->bins[which];
+  SE_TRY(slot_alloc2d(ctx, SE_SLOT_RAW, Cout, X.cols));
+  SE_TRY(slot_alloc2d(ctx, SE_SLOT_PROB, Cout, X.cols));
+  SE_TRY(slot_alloc2d(ctx, SE_SLOT_LABEL, 1, X.cols));
+  const SlotBuf& R = ctx->slot[SE_SLOT_RAW];
+  if (ctx->forest_leaves_cap < lv.size()) {
+    if (ctx->d_forest_leaves) cudaFree(ctx->d_forest_leaves);
+    ctx->d_forest_leaves = nullptr; ctx->forest_leaves_cap = 0;
+    SE_CUDA(ctx, cudaMalloc(&ctx->d_forest_leaves, sizeof(float) * lv.size()));
+    ctx->forest_leaves_cap = lv.size();
+  }
+  SE_CUDA(ctx, cudaMemcpyAsync(ctx->d_forest_leaves, lv.data(), sizeof(float) * lv.size(), cudaMemcpyHostToDevice, ctx->stream));
+  ForestClassArgs a;
+  a.X8 = B.d8; a.n = X.cols; a.ld8 = B.ld8;
+  a.mode = mode; a.K = K;
+  a.leaves = ctx->d_forest_leaves;
+  a.raw = R.d; a.ld_raw = Cout > 1 ? R.ld : R.cols;
+  std::vector<int32_t> local((size_t)X.rows, -1);
+  std::vector<int32_t> used;
+  std::vector<unsigned char> blob;
+  int chunks = 0, p0 = 0, prev_last = -1;
+  while (p0 < n_trees) {
+    size_t nodes = 0;
+    const int p1 = forest_chunk(order.data(), p0, n_trees, offsets, feature, local, used, nodes, forest_classify_bytes);
+    SE_REQUIRE(ctx, p1 > p0, SE_ERR_ARG, "tree %d alone (%d nodes) does not fit the forest kernel's shared memory", order[p0],
+               offsets[order[p0] + 1] - offsets[order[p0]]);
+    const size_t T = (size_t)(p1 - p0), C = used.size(), Nn = nodes;
+    // classes this chunk writes, and which of them continue a sum an earlier chunk left in RAW
+    a.c0 = gbm ? order[p0] % dim : 0;
+    a.c1 = gbm ? order[p1 - 1] % dim + 1 : S;
+    a.acc0 = a.c0;
+    a.acc1 = gbm ? (a.c0 == prev_last ? a.c0 + 1 : a.c0) : (chunks > 0 ? S : 0);
+    const size_t NC = gbm ? (size_t)(a.c1 - a.c0) : 0;
+    a.T = (int)T; a.C = (int)C;
+    a.off_init = (int)(8 * T);
+    a.off_coloff = a.off_init + (int)(8 * NC);
+    a.off_nodes = a.off_coloff + (int)(8 * C);
+    a.off_treeoff = a.off_nodes + (int)(8 * Nn);
+    a.off_lbase = a.off_treeoff + (int)(4 * (T + 1));
+    a.off_cstart = a.off_lbase + (int)(4 * T);
+    a.blob_bytes = (int)pad_to((size_t)a.off_cstart + 4 * (NC + 1), 16);
+    a.off_ranks = a.blob_bytes;
+    a.off_parked = a.off_ranks + (int)pad_to(C * kForestTile, 16);
+    blob.assign((size_t)a.blob_bytes, 0);
+    double* bw = reinterpret_cast<double*>(blob.data());
+    double* binit = reinterpret_cast<double*>(blob.data() + a.off_init);
+    unsigned long long* bco = reinterpret_cast<unsigned long long*>(blob.data() + a.off_coloff);
+    uint2* bn = reinterpret_cast<uint2*>(blob.data() + a.off_nodes);
+    int32_t* bto = reinterpret_cast<int32_t*>(blob.data() + a.off_treeoff);
+    int32_t* blb = reinterpret_cast<int32_t*>(blob.data() + a.off_lbase);
+    int32_t* bcs = reinterpret_cast<int32_t*>(blob.data() + a.off_cstart);
+    for (size_t c = 0; c < C; ++c) bco[c] = (unsigned long long)used[c] * (unsigned long long)B.ld8;
+    for (size_t j = 0; j < NC; ++j) binit[j] = init ? init[a.c0 + j] : 0.0;
+    size_t at = 0;
+    for (int p = p0; p < p1; ++p) {
+      const int t = order[p];
+      const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
+      bw[p - p0] = weights ? weights[t] : 1.0;  // GBM: weights[t] = a(t / dim)(t % dim); SAMME: a_t
+      bto[p - p0] = (int32_t)at;
+      blb[p - p0] = lbase[t];
+      forest_pack_tree(B, local, b, nn, feature, threshold, left, right, bn + at);
+      at += (size_t)nn;
+      if (gbm) bcs[t % dim - a.c0 + 1] = p - p0 + 1;  // trees of class c: [cstart[c - c0], cstart[c - c0 + 1])
+    }
+    bto[T] = (int32_t)at;
+    SE_TRY(forest_upload_blob(ctx, blob));
+    a.blob = ctx->d_forest;
+    SE_LAUNCH_T(ctx, SE_KF_TREE, launch_forest_classify(a, ctx->sms, ctx->stream));
+    ++chunks;
+    prev_last = a.c1 - 1;
+    p0 = p1;
+  }
+  SE_LAUNCH_T(ctx, SE_KF_AGG, launch_agg_finalize(kind, Cout, K, dim, loss, M, sum_a, X.cols, a.ld_raw, R.d,
+                                                  ctx->slot[SE_SLOT_PROB].d, ctx->slot[SE_SLOT_LABEL].d, ctx->sms,
+                                                  ctx->stream));
   ctx->last_forest_chunks = chunks;
   ctx->last_tree_binned = 1;
   return end(ctx);

@@ -265,6 +265,40 @@ struct ForestArgs {
 constexpr int kForestTile = 256;              // rows per CTA tile (one row per thread)
 constexpr int kForestSmemBudget = 54 * 1024;  // per CTA: four CTAs per SM (the walk is latency-bound: warps matter more than chunk size)
 cudaError_t launch_forest_predict(const ForestArgs& a, int sms, cudaStream_t s);
+// A classifier ensemble in ONE pass over the uint8 rank matrix: the stage-1 class sums of the aggregation (what
+// agg_finalize reads from RAW) for classes [c0, c1), RAW[c][row] = start_c + Σ_t w_t · leaf contribution, fp64 in model
+// order; start_c = RAW[c][row] for c in [acc0, acc1) (a sum an earlier chunk began), else init_c (GBM) or 0.
+// Leaf kinds (mode): one value per leaf for the tree's own class (GBM: trees of class c are [cstart[c-c0], cstart[c-c0+1]));
+// K values per leaf (class probabilities, or their logs for SAMME.R); a label per leaf (a vote of weight w_t).
+// `blob` (copied verbatim into shared memory):
+//   [0)            double   w[T]
+//   [off_init)     double   init of classes c0.. (GBM only)
+//   [off_coloff)   uint64   byte offset of local column c in X8 (column * ld8), c < C
+//   [off_nodes)    uint2    nodes as in ForestArgs, a leaf's y = its ordinal among the tree's leaves
+//   [off_treeoff)  int32    first node of tree t (T + 1 entries)
+//   [off_lbase)    int32    first value of tree t's leaves in `leaves`
+//   [off_cstart)   int32    GBM: first tree of class c0 + j (c1 - c0 + 1 entries)
+//   [off_ranks)    uint8    (shared memory only) the tile's ranks, [C][256]
+//   [off_parked)   uint16   (shared memory only) leaf ordinal (label for label leaves) per tree and row, [T][256]
+enum { kForestScalarLeaves = 0, kForestVectorLeaves = 1, kForestLabelLeaves = 2 };
+struct ForestClassArgs {
+  const uint8_t* X8 = nullptr;
+  int64_t n = 0, ld8 = 0;
+  const unsigned char* blob = nullptr;
+  int blob_bytes = 0;  // multiple of 16
+  int T = 0, C = 0;
+  int off_init = 0, off_coloff = 0, off_nodes = 0, off_treeoff = 0, off_lbase = 0, off_cstart = 0, off_ranks = 0, off_parked = 0;
+  int mode = 0, K = 0;
+  int c0 = 0, c1 = 0, acc0 = 0, acc1 = 0;
+  const float* leaves = nullptr;  // device leaf table
+  float* raw = nullptr;           // [C][ld_raw]
+  int64_t ld_raw = 0;
+};
+cudaError_t launch_forest_classify(const ForestClassArgs& a, int sms, cudaStream_t s);
+// The classifier aggregations' epilogue (se_agg.cu agg_finalize_kernel) over the stage-1 sums already in raw[C][ld]:
+// raw, prob and label as se_agg_run writes them.  M: members (bagging: prob = raw / M); sum_a: Σ a_m (SAMME).
+cudaError_t launch_agg_finalize(int kind, int C, int K, int dim, int loss, int M, double sum_a, int64_t n, int64_t ld,
+                                float* raw, float* prob, float* label, int sms, cudaStream_t s);
 cudaError_t launch_linear_predict(const float* X, int64_t n, int64_t ld, int n_coef,
                                   const float* coef, const int32_t* cols, float intercept,
                                   float* out, int sms, cudaStream_t s);

@@ -387,6 +387,101 @@ __global__ void __launch_bounds__(kForestTile) forest_predict_kernel(const Fores
   }
 }
 
+// The same tile for classifier ensembles.  Phase 1: every thread walks every tree of the chunk for its row (two walks
+// in flight) and parks the leaf's ordinal — or, for label leaves, the label itself — in shared memory, [T][256] uint16.
+// Phase 2: the classes are swept kClassGroup at a time with fp64 accumulators in registers, each adding the trees in
+// model order (the reference's loop order), and every class sum leaves as one coalesced row store into RAW[c].  Class
+// probabilities come from the leaf table in global memory (K floats per leaf: L1/L2-resident for realistic forests),
+// so neither K nor the class range of a chunk costs shared memory.
+constexpr int kClassGroup = 4;
+
+template <int MODE>
+__global__ void __launch_bounds__(kForestTile, 2) forest_classify_kernel(const ForestClassArgs a) {
+  extern __shared__ __align__(16) unsigned char fsm[];
+  for (int i = threadIdx.x; i < a.blob_bytes / 16; i += kForestTile)
+    reinterpret_cast<uint4*>(fsm)[i] = __ldg(reinterpret_cast<const uint4*>(a.blob) + i);
+  const double* s_w = reinterpret_cast<const double*>(fsm);
+  const double* s_init = reinterpret_cast<const double*>(fsm + a.off_init);
+  const unsigned long long* s_coloff = reinterpret_cast<const unsigned long long*>(fsm + a.off_coloff);
+  const uint2* s_nodes = reinterpret_cast<const uint2*>(fsm + a.off_nodes);
+  const int* s_toff = reinterpret_cast<const int*>(fsm + a.off_treeoff);
+  const int* s_lbase = reinterpret_cast<const int*>(fsm + a.off_lbase);
+  const int* s_cstart = reinterpret_cast<const int*>(fsm + a.off_cstart);
+  unsigned char* s_rank = fsm + a.off_ranks;
+  uint16_t* s_park = reinterpret_cast<uint16_t*>(fsm + a.off_parked) + threadIdx.x;  // this thread's column
+  const int64_t ntiles = (a.n + kForestTile - 1) / kForestTile;
+  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    __syncthreads();  // the packed trees are staged (first tile) / the previous tile's ranks are no longer read
+    const int64_t row0 = tile * kForestTile;
+    for (int i = threadIdx.x; i < a.C * (kForestTile / 4); i += kForestTile) {
+      const int c = i / (kForestTile / 4), q = i % (kForestTile / 4);
+      const int64_t r = row0 + 4 * q;  // columns are padded to 128 rows: a word at r < ld8 stays inside its column
+      uint32_t v = 0;
+      if (r < a.ld8) v = __ldg(reinterpret_cast<const uint32_t*>(a.X8 + s_coloff[c] + r));
+      *reinterpret_cast<uint32_t*>(s_rank + c * kForestTile + 4 * q) = v;
+    }
+    __syncthreads();
+    const int64_t row = row0 + threadIdx.x;
+    if (row >= a.n) continue;  // no barrier below: a thread only reads back what it parked itself
+    const unsigned char* myr = s_rank + threadIdx.x;
+    auto park = [&](int t, int d) {
+      const uint32_t ord = s_nodes[s_toff[t] + d].y;
+      s_park[t * kForestTile] =
+          (MODE == kForestLabelLeaves) ? (uint16_t)__float2uint_rz(__ldg(a.leaves + s_lbase[t] + ord)) : (uint16_t)ord;
+    };
+    int t = 0;
+    for (; t + 1 < a.T; t += 2) {  // two independent walks in flight
+      const uint2* n0 = s_nodes + s_toff[t];
+      const uint2* n1 = s_nodes + s_toff[t + 1];
+      int d0 = 0, d1 = 0;
+      bool l0 = true, l1 = true;
+      while (l0 || l1) {
+        if (l0) forest_step(n0, myr, d0, l0);
+        if (l1) forest_step(n1, myr, d1, l1);
+      }
+      park(t, d0);
+      park(t + 1, d1);
+    }
+    if (t < a.T) {
+      int d0 = 0;
+      bool l0 = true;
+      while (l0) forest_step(s_nodes + s_toff[t], myr, d0, l0);
+      park(t, d0);
+    }
+    float* out = a.raw + row;
+    if (MODE == kForestScalarLeaves) {  // GBM: class c sums its own trees, init_c + Σ_i a_ic · tree_ic(x)
+      for (int c = a.c0; c < a.c1; ++c) {
+        double acc = (c >= a.acc0 && c < a.acc1) ? (double)out[(int64_t)c * a.ld_raw] : s_init[c - a.c0];
+        for (int u = s_cstart[c - a.c0]; u < s_cstart[c - a.c0 + 1]; ++u)
+          acc += s_w[u] * (double)__ldg(a.leaves + s_lbase[u] + s_park[u * kForestTile]);
+        out[(int64_t)c * a.ld_raw] = (float)acc;
+      }
+    } else {
+      for (int c = a.c0; c < a.c1; c += kClassGroup) {
+        double acc[kClassGroup];
+#pragma unroll
+        for (int j = 0; j < kClassGroup; ++j)
+          acc[j] = (c + j < a.c1 && c + j >= a.acc0 && c + j < a.acc1) ? (double)out[(int64_t)(c + j) * a.ld_raw] : 0.0;
+        for (int u = 0; u < a.T; ++u) {
+          const int v = s_park[u * kForestTile];
+          if (MODE == kForestLabelLeaves) {  // a vote of weight w_u for class v
+#pragma unroll
+            for (int j = 0; j < kClassGroup; ++j) acc[j] += (v == c + j) ? s_w[u] : 0.0;
+          } else {  // the leaf's class vector, this group's slice
+            const float* lv = a.leaves + s_lbase[u] + (int64_t)v * a.K + c;
+#pragma unroll
+            for (int j = 0; j < kClassGroup; ++j)
+              if (c + j < a.c1) acc[j] += s_w[u] * (double)__ldg(lv + j);
+          }
+        }
+#pragma unroll
+        for (int j = 0; j < kClassGroup; ++j)
+          if (c + j < a.c1) out[(int64_t)(c + j) * a.ld_raw] = (float)acc[j];
+      }
+    }
+  }
+}
+
 constexpr int LU = 8;
 
 __global__ void __launch_bounds__(kBlock) linear_predict_kernel(const float* __restrict__ X, int64_t n,
@@ -517,6 +612,26 @@ cudaError_t launch_forest_predict(const ForestArgs& a, int sms, cudaStream_t st)
   if (need < 1) need = 1;
   const int64_t cap = (int64_t)sms * per_sm;
   forest_predict_kernel<<<(int)(need < cap ? need : cap), kForestTile, smem, st>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_forest_classify(const ForestClassArgs& a, int sms, cudaStream_t st) {
+  const size_t smem = (size_t)a.off_parked + (size_t)a.T * kForestTile * sizeof(uint16_t);
+  if (a.T < 1 || a.C < 0 || smem > 220 * 1024 || (a.blob_bytes & 15) != 0 || (a.off_parked & 15) != 0) return cudaErrorInvalidValue;
+  auto kern = a.mode == kForestScalarLeaves   ? forest_classify_kernel<kForestScalarLeaves>
+              : a.mode == kForestVectorLeaves ? forest_classify_kernel<kForestVectorLeaves>
+                                              : forest_classify_kernel<kForestLabelLeaves>;
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  int per_sm = (int)((220 * 1024) / (smem + 1024));
+  if (per_sm < 1) per_sm = 1;
+  if (per_sm > 8) per_sm = 8;
+  int64_t need = (a.n + kForestTile - 1) / kForestTile;
+  if (need < 1) need = 1;
+  const int64_t cap = (int64_t)sms * per_sm;
+  kern<<<(int)(need < cap ? need : cap), kForestTile, smem, st>>>(a);
   return cudaGetLastError();
 }
 

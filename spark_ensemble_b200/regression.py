@@ -59,6 +59,40 @@ def _split_validation(est: Params, dataset: DataFrame):
     return dataset, None
 
 
+# Param `forestTransform` of the tree-ensemble models: transform evaluates the whole forest in one pass over the
+# feature matrix on the device (se_forest_predict / se_forest_classify) instead of predicting every member on the host
+# and aggregating the stacked outputs.  Off by default.
+_pforest = [Param("forestTransform", "transform tree ensembles in one pass over the device-resident features", convert=bool)]
+
+
+def _member_trees(models):
+    """tree_arrays() of every member, or None when there is none or one is not a tree."""
+    trees = [m.tree_arrays() for m in models]
+    return trees if trees and all(t is not None for t in trees) else None
+
+
+def _forest_transform(device: int, X, run):
+    """Uploads X column-major once and returns run(ctx); None when the rank matrix cannot hold the forest (SE_ERR_STATE:
+    a column with more than 255 distinct thresholds), so that the caller takes the member-by-member route."""
+    X = np.asarray(X, dtype=np.float32)
+    with Context(device) as ctx:
+        ctx.alloc(N.SLOT_X, X.shape[1], X.shape[0])
+        ctx.upload_rowmajor(N.SLOT_X, X)
+        try:
+            return run(ctx)
+        except N.NativeError as e:
+            if e.code != N.SE_ERR_STATE:
+                raise
+            return None
+
+
+def _forest_predict(ctx: Context, trees, subspaces, weights, init: float) -> np.ndarray:
+    n = ctx.layout(N.SLOT_X)[1]
+    ctx.alloc(N.SLOT_RAW, 1, n)
+    ctx.forest_predict(trees, N.SLOT_RAW, weights=weights, init=init, subspaces=subspaces)
+    return ctx.download(N.SLOT_RAW).astype(np.float64)
+
+
 class GBMRegressor(Params):
     """regression/GBMRegressor.scala:164-476.  UID prefix "GBMRegressor2" (sic, :229)."""
 
@@ -195,9 +229,9 @@ _preg = [
           lambda v: [int(d) for d in v]),
 ]
 _GBM_REG_DEFAULTS = {**_d, **_ds, **_db, **_dg, "loss": "squared", "alpha": 0.9, "initStrategy": "constant", "residentFeatures": False, "lineSearch": "brent",
-                     "devices": [],
+                     "devices": [], "forestTransform": False,
                      "seed": java_string_hash("org.apache.spark.ml.regression.GBMRegressor")}
-GBMRegressor._declare(_p + _ps + _pb + _pg + _preg, _GBM_REG_DEFAULTS)
+GBMRegressor._declare(_p + _ps + _pb + _pg + _preg + _pforest, _GBM_REG_DEFAULTS)
 
 
 def _stack_model_outputs(models, subspaces, X, extra=None) -> np.ndarray:
@@ -225,6 +259,12 @@ class GBMRegressionModel(Params):
     def _aggregate(self, X) -> np.ndarray:
         n = X.shape[0]
         const_init = hasattr(self.init, "prediction")
+        trees = _member_trees(self.models) if self("forestTransform") and const_init else None
+        if trees is not None:
+            out = _forest_transform(self.device, X, lambda ctx: _forest_predict(ctx, trees, self.subspaces, self.weights,
+                                                                                self.init.prediction))
+            if out is not None:
+                return out
         P = _stack_model_outputs(self.models, self.subspaces, X,
                                  None if const_init else self.init.predict(X))
         a = self.weights if const_init else np.concatenate([[1.0], self.weights])
@@ -243,7 +283,7 @@ class GBMRegressionModel(Params):
         return float(self._aggregate(np.asarray(features).reshape(1, -1))[0])
 
 
-GBMRegressionModel._declare(_p + _ps + _pb + _pg + _preg, _GBM_REG_DEFAULTS)
+GBMRegressionModel._declare(_p + _ps + _pb + _pg + _preg + _pforest, _GBM_REG_DEFAULTS)
 
 
 # ---- Bagging (train is out of the hot path: embarrassingly parallel base-learner fits) ---------------
@@ -281,9 +321,9 @@ _pbag = [Param("numBaseLearners", "number of base learners", ParamValidators.gtE
          Param("baseLearner", "base learner"),
          Param("parallelism", "the number of threads to use when running parallel algorithms (>= 1)",
                ParamValidators.gtEq(1), int)]
-_BAG_REG_DEFAULTS = {**_d, **_ds, "numBaseLearners": 10, "parallelism": 1,
+_BAG_REG_DEFAULTS = {**_d, **_ds, "numBaseLearners": 10, "parallelism": 1, "forestTransform": False,
                      "seed": java_string_hash("org.apache.spark.ml.regression.BaggingRegressor")}
-BaggingRegressor._declare(_p + _ps + _pbag, _BAG_REG_DEFAULTS)
+BaggingRegressor._declare(_p + _ps + _pbag + _pforest, _BAG_REG_DEFAULTS)
 
 
 class BaggingRegressionModel(Params):
@@ -297,6 +337,12 @@ class BaggingRegressionModel(Params):
         self.parent = None
 
     def _aggregate(self, X) -> np.ndarray:
+        trees = _member_trees(self.models) if self("forestTransform") else None
+        if trees is not None:  # (Σ_i m_i) / M as Σ_i m_i / M
+            out = _forest_transform(self.device, X, lambda ctx: _forest_predict(
+                ctx, trees, self.subspaces, np.full(len(trees), 1.0 / len(trees)), 0.0))
+            if out is not None:
+                return out
         P = _stack_model_outputs(self.models, self.subspaces, X)
         with Context(self.device) as ctx:
             ctx.agg_configure(N.AGG_BAGGING_REGRESSOR, P.shape[0], 0, 1, 0, X.shape[0])
@@ -311,7 +357,7 @@ class BaggingRegressionModel(Params):
         return float(self._aggregate(np.asarray(features).reshape(1, -1))[0])
 
 
-BaggingRegressionModel._declare(_p + _ps + _pbag, _BAG_REG_DEFAULTS)
+BaggingRegressionModel._declare(_p + _ps + _pbag + _pforest, _BAG_REG_DEFAULTS)
 
 
 # ---- BoostingRegressor (AdaBoost.R2, Drucker 1997): SURVEY.md §8f-2 -----------------------------------

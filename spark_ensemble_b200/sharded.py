@@ -20,6 +20,7 @@ from .ensemble import row_partition
 
 _TRAIN_SLOTS = {N.SLOT_Y, N.SLOT_W, N.SLOT_F, N.SLOT_H, N.SLOT_R, N.SLOT_WOUT, N.SLOT_BAG, N.SLOT_X}
 _VALID_SLOTS = {N.SLOT_VY, N.SLOT_VF, N.SLOT_VH, N.SLOT_VX}
+_OUT_SLOTS = {N.SLOT_RAW, N.SLOT_PROB, N.SLOT_LABEL}
 
 
 class ShardedContext:
@@ -31,7 +32,7 @@ class ShardedContext:
         self.world = len(devices)
         self.ctxs = [context_factory(d) for d in devices]
         self._pool = cf.ThreadPoolExecutor(max_workers=self.world)
-        self.n = self.nv = 0
+        self.n = self.nv = self._n_out = 0
         self.dim = 1
         if join:
             uid = Context.comm_unique_id()
@@ -47,6 +48,8 @@ class ShardedContext:
             return self.n
         if slot in _VALID_SLOTS:
             return self.nv
+        if slot in _OUT_SLOTS:  # the outputs of forest_classify: one column per row of the feature slot it read
+            return self._n_out
         raise ValueError(f"slot {slot} is not row-sharded by ShardedContext")
 
     def close(self):
@@ -214,6 +217,13 @@ class ShardedContext:
     def forest_predict(self, trees, out_slot, weights=None, init=0.0, out_row=0, validation=False, subspaces=None):
         self._all(lambda r, c: c.forest_predict(trees, out_slot, weights=weights, init=init, out_row=out_row,
                                                 validation=validation, subspaces=subspaces))
+
+    def forest_classify(self, trees, kind, num_classes, dim=1, loss=0, weights=None, init=None, validation=False,
+                        subspaces=None):
+        """Every shard classifies its own rows (no reduction): RAW / PROB / LABEL reassemble through `download`."""
+        self._n_out = self.nv if validation else self.n
+        self._all(lambda r, c: c.forest_classify(trees, kind, num_classes, dim=dim, loss=loss, weights=weights, init=init,
+                                                 validation=validation, subspaces=subspaces))
 
     def linear_predict(self, coef, intercept, out_slot, out_row=0, validation=False, subspace=None):
         self._all(lambda r, c: c.linear_predict(coef, intercept, out_slot, out_row, validation=validation, subspace=subspace))
