@@ -351,6 +351,24 @@ SE_API int se_forest_classify(se_ctx* ctx, int which, int kind, int num_classes,
                               int n_trees, const int32_t* offsets, const int32_t* feature, const float* threshold,
                               const int32_t* left, const int32_t* right, const float* leaf, int leaf_width,
                               const double* weights, const double* init);
+/* AdaBoost.R2's weighted median of tree members in ONE pass over the uint8 rank matrix of X (which = 0) or VX (which = 1):
+ * row out_row of out_slot receives Utils.weightedMedian([tree_t(x)]_t, weights) for every row, with no [M][n] member
+ * outputs.  Trees are concatenated as in se_forest_predict (offsets, tree-local children, GLOBAL columns, `value` = the
+ * leaf value per node), in model order; equal member values are ordered by model index (the reference's stable sortBy).
+ * The output is bit-identical to se_tree_predict of every member into row t of SE_SLOT_P followed by
+ * se_agg_configure(SE_AGG_BOOSTING_REG_MEDIAN, M, ...) + se_agg_run(weights), for every weight vector (zero, negative,
+ * equal, half-weight ties) and with option wm_fast on or off: it is a selection among the fp32 leaf values.  The weights
+ * choose the mode exactly as in se_agg_run (last_wm_mode: 0 exact, 1 fast + margin, 2 equal weights); in mode 1 the rows
+ * inside the rounding margin take the exact pick in the same thread and last_wm_deferred counts them.
+ * Sets last_forest_chunks = 1 and last_tree_binned = 1.
+ * SE_ERR_ARG: a null pointer (weights included), a node array that is not a tree, a column outside X.
+ * SE_ERR_STATE: no feature slot, an output slot whose column count differs from the feature slot's, a column that needs
+ * more than 255 thresholds, more than 64 trees, or a forest that does not fit ONE chunk of the forest kernel's shared
+ * memory (nodes, leaf values, ranks and parked leaves within 216 KB) — evaluate the members with se_tree_predict +
+ * se_agg_run then. */
+SE_API int se_forest_weighted_median(se_ctx* ctx, int which, int n_trees, const int32_t* offsets, const int32_t* feature,
+                                     const float* threshold, const int32_t* left, const int32_t* right, const float* value,
+                                     const double* weights, int out_slot, int out_row);
 /* linear model: out = intercept + Σ_j coef[j]·X[subspace[j]] */
 SE_API int se_linear_predict(se_ctx* ctx, int which, int n_coef, const float* coef, float intercept,
                       const int32_t* subspace, int out_slot, int out_row);

@@ -116,6 +116,11 @@ TABLE = [
                                               ("threshold", "in_f32"), ("left", "in_i32"), ("right", "in_i32"), ("leaf", "in_f32"),
                                               ("leafWidth", "i32"), ("weights", "in_f64"), ("init", "in_f64")],
      "predictRaw / probability / prediction of a classifier ensemble of tree members in one pass: RAW, PROB, LABEL slots"),
+    ("forestWeightedMedian", "se_forest_weighted_median", [("ctx", "ctx"), ("which", "i32"), ("nTrees", "i32"), ("offsets", "in_i32"),
+                                                           ("feature", "in_i32"), ("threshold", "in_f32"), ("left", "in_i32"),
+                                                           ("right", "in_i32"), ("value", "in_f32"), ("weights", "in_f64"),
+                                                           ("outSlot", "i32"), ("outRow", "i32")],
+     "BoostingRegressionModel.predict (median) for tree members: weighted median of tree(x) in one pass"),
     ("linearPredict", "se_linear_predict", [("ctx", "ctx"), ("which", "i32"), ("nCoef", "i32"), ("coef", "in_f32"), ("intercept", "f32"),
                                             ("subspace", "in_i32"), ("outSlot", "i32"), ("outRow", "i32")], ""),
 ]

@@ -114,6 +114,7 @@ PROTOTYPES = {
     "se_tree_predict_multi": [_vp, _i32, _i32, _ip, _fp, _ip, _ip, _fp, _i32, _ip, _i32, _i32],
     "se_forest_predict": [_vp, _i32, _i32, _ip, _ip, _fp, _ip, _ip, _fp, _dp, _d, _i32, _i32],
     "se_forest_classify": [_vp, _i32, _i32, _i32, _i32, _i32, _i32, _ip, _ip, _fp, _ip, _ip, _fp, _i32, _dp, _dp],
+    "se_forest_weighted_median": [_vp, _i32, _i32, _ip, _ip, _fp, _ip, _ip, _fp, _dp, _i32, _i32],
     "se_linear_predict": [_vp, _i32, _i32, _fp, _f, _ip, _i32, _i32],
 }
 _RESTYPES = {"se_last_error": C.c_char_p}

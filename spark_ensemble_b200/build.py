@@ -20,7 +20,7 @@ LIB = os.path.join(LIBDIR, "libse_b200.so")
 SOURCES = ["se_api.cu", "se_gbm.cu", "se_gbm_tiled.cu", "se_gbm_fused.cu", "se_gbm_generic.cu", "se_brent.cu", "se_boost.cu", "se_agg.cu", "se_models.cu", "se_util.cu"]
 # the device Brent must round every multiply and add separately to reproduce the host line search bit for bit
 EXTRA_FLAGS = {"se_brent.cu": ["-fmad=false"], "se_gbm_fused.cu": ["-fmad=false"]}
-HEADERS = ["se_common.cuh", "se_kernels.h", "se_loss.cuh", "se_tma.cuh", "se_brent.h", "se_sortnet.h", os.path.join("..", "..", "include", "se_abi.h")]
+HEADERS = ["se_common.cuh", "se_kernels.h", "se_loss.cuh", "se_tma.cuh", "se_brent.h", "se_sortnet.h", "se_wmedian.cuh", os.path.join("..", "..", "include", "se_abi.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

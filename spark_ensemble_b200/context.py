@@ -429,6 +429,20 @@ class Context:
                                               N.fptr(v), int(width), None if w is None else N.dptr(w),
                                               None if i is None else N.dptr(i)))
 
+    def forest_weighted_median(self, trees, out_slot: int, weights, out_row: int = 0, validation: bool = False):
+        """out = Utils.weightedMedian([tree_t(x)]_t, weights) for a list of at most 64 regression trees (dicts as in
+        tree_predict, features = columns of X, model order) in one pass over the resident feature matrix
+        (se_forest_weighted_median: BoostingRegressionModel.predict, regression/BoostingRegressor.scala:333-337).  The
+        same bits as tree_predict of every member + agg_run(AGG_BOOSTING_REG_MEDIAN); NativeError SE_ERR_STATE when
+        the forest is beyond the kernel (more than 64 trees, more than one chunk, a column with > 255 thresholds)."""
+        offs, f, t, l, r, v = _flatten_trees(trees, None, "value")
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64).reshape(-1)
+        if w is not None and w.size != len(trees):
+            raise ValueError("one weight per tree")
+        self._ck(self._lib.se_forest_weighted_median(self._h, int(validation), len(trees), N.iptr(offs), N.iptr(f),
+                                                     N.fptr(t), N.iptr(l), N.iptr(r), N.fptr(v),
+                                                     None if w is None else N.dptr(w), out_slot, out_row))
+
     def linear_predict(self, coef, intercept: float, out_slot: int, out_row: int = 0,
                        validation: bool = False, subspace=None):
         c = np.ascontiguousarray(coef, dtype=np.float32)

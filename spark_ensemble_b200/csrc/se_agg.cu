@@ -17,6 +17,7 @@
 #include "se_loss.cuh"
 #include "se_tma.cuh"
 #include "se_sortnet.h"
+#include "se_wmedian.cuh"
 #include "../../include/se_abi.h"
 
 namespace se {
@@ -541,14 +542,6 @@ __global__ void __launch_bounds__(kBlock) agg_finalize_kernel(const FinArgs f) {
 // whole warp, O(M log² M) compare-exchanges instead of the O(M²) threshold scan it replaces (which was 0.07 of the
 // HBM roofline at M = 32 because per-lane pruning diverges).  Total and running sums are then accumulated in fp64 in
 // sorted order, exactly like the reference.
-__device__ __forceinline__ uint32_t wm_key(float x) {
-  const uint32_t u = __float_as_uint(x + 0.0f);  // -0 -> +0: equal values stay ties
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float wm_unkey(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
-
 template <int T>
 __global__ void __launch_bounds__(T) agg_wmedian_kernel(const float* __restrict__ P, int64_t n, int64_t ld, int M,
                                                        int Mp, const double* __restrict__ a,
@@ -660,35 +653,6 @@ __global__ void __launch_bounds__(32 * kWmWarps) agg_wmedian_warp_kernel(const f
   }
 }
 
-// sort of the (key, model) words + the reference's sorted-order cumulative sums (ensemble/Utils.scala:31-38)
-template <int MP>
-__device__ __forceinline__ unsigned long long wm_exact_pick(unsigned long long (&w)[MP], int M, const double* s_a) {
-  sortnet_oddeven<MP>(w, [](unsigned long long& x, unsigned long long& y) {
-    const bool swap = x > y;
-    const unsigned long long lo = swap ? y : x, hi = swap ? x : y;
-    x = lo;
-    y = hi;
-  });
-  double total = 0.0;
-#pragma unroll
-  for (int m = 0; m < MP; ++m)
-    if (m < M) total += s_a[(unsigned)w[m]];
-  const double half = 0.5 * total;
-  double cum = 0.0;
-  bool found = false;
-  unsigned long long pick = 0ull;
-#pragma unroll
-  for (int m = 0; m < MP; ++m) {
-    if (m < M) {
-      cum += s_a[(unsigned)w[m]];
-      const bool hit = !found && (cum >= half);
-      pick = (hit || (!found && m == M - 1)) ? w[m] : pick;  // last element when nothing reaches half (NaN weights)
-      found = found || hit;
-    }
-  }
-  return pick;
-}
-
 // Same algorithm with the row's words in REGISTERS (Mp <= 64): the network is fully unrolled, so every
 // compare-exchange is ~6 ALU instructions and no memory traffic — the shared-memory form above moves 32 B per
 // compare-exchange and thread and is bound by shared-memory bandwidth (measured 8.0 ms for 25 M rows at M = 32).
@@ -737,33 +701,7 @@ __global__ void __launch_bounds__(128) agg_wmedian_reg_kernel(const __grid_const
   }
 }
 
-// ---- weighted median, fast path (M <= 64, all weights finite and >= 0) -------------------------------------------
-// The exact kernels above carry (key, model) words through the sort because the reference accumulates the weights in
-// SORTED order (ensemble/Utils.scala:31-38) — 6 ALU-pipe instructions per compare-exchange, and the ALU pipe issues at
-// half rate: 4.07 ms for 25 M rows x 32 models.  With weights >= 0 the answer is `the smallest value v whose group-end
-// cumulative weight C(v) reaches h = total / 2` (cumulative sums are monotone in fp64 too).  C(v) and h are recursive
-// fp64 sums of the same addends as Ĉ(v) = Σ_{x_j <= v} a_j and ĥ = T̂ / 2 taken in MODEL order, so
-//     |(C(v) - h) - (Ĉ(v) - ĥ)| <= 3 (M - 1) 2^-53 T (1 + eps)
-// and whenever both neighbours of the crossing clear the margin tau = 8 M 2^-53 T̂ the model-order decision IS the
-// reference's decision.  So: sort the 32-bit keys alone (min/max, 2 instructions per compare-exchange, Batcher's
-// 191-element network), bisect the sorted keys on Ĉ (5 x 32 predicated DADDs with the weights as constant-bank
-// operands), and send the rows that do not clear the margin — none for generic weights, the exact ties for
-// small-integer weights — to the exact kernel through a compacted list (mode 2: all weights equal, where both orders
-// produce the same sums and no margin is needed).
-struct WmWeights {
-  double w[64];
-};
-
-template <int MP, int L>
-__device__ __forceinline__ uint32_t wm_candidate(const uint32_t (&s)[MP], uint32_t t) {
-  // level-L bisection probe: position step - 1 + t * 2 * step, t in [0, 2^L) — a select tree over static indices
-  constexpr int step = MP >> (L + 1);
-  uint32_t v = s[step - 1];
-#pragma unroll
-  for (int q = 1; q < (1 << L); ++q) v = (t == (uint32_t)q) ? s[step - 1 + q * 2 * step] : v;
-  return v;
-}
-
+// ---- weighted median, fast path (M <= 64, all weights finite and >= 0): see se_wmedian.cuh ---------------------
 template <int MP>
 __global__ void __launch_bounds__(128) agg_wmedian_fast_kernel(const __grid_constant__ CUtensorMap mapP, int64_t n, int M,
                                                                const __grid_constant__ WmWeights wts, double total,
@@ -981,13 +919,9 @@ cudaError_t launch_agg(const AggArgs& a, int ctas_per_sm, int sms, cudaStream_t 
         if (a.wm_mode != 0 && a.weights64_host != nullptr && (a.wm_mode == 2 || (a.wm_list != nullptr && a.wm_count != nullptr))) {
           // fast path: keys-only sort + model-order sums; rows inside the rounding margin go to the exact list kernel
           WmWeights wts;
-          double total = 0.0;
-          for (int m = 0; m < 64; ++m) {
-            wts.w[m] = (m < a.M) ? a.weights64_host[m] : 0.0;
-            total += wts.w[m];  // model order, like the kernel's own sums
-          }
+          double total = 0.0, tau = 0.0;
+          wm_fast_operands(a.weights64_host, a.M, a.wm_mode, &wts, &total, &tau);
           const bool margin = (a.wm_mode == 1);
-          const double tau = margin ? 8.0 * (double)a.M * 1.1102230246251565e-16 * total : -1.0;  // mode 2: every row is safe
           const size_t fsmem = 2 * (size_t)a.M * 128 * sizeof(float) + 128;
           if (margin) {
             e = cudaMemsetAsync(a.wm_count, 0, sizeof(unsigned int), st);

@@ -2741,10 +2741,11 @@ size_t pad_to(size_t v, size_t to) { return (v + to - 1) / to * to; }
 // Grows the chunk of trees order[p0..p1) (order == nullptr: identity) tree by tree while bytes(trees, columns, nodes),
 // the kernel's shared memory, fits the budget; a member that does not fit the four-CTAs-per-SM budget alone gets two,
 // then one CTA per SM.  On return `used` lists the chunk's global columns and local[] maps them to their position.
-// Returns p1 (== p0: even one tree does not fit).
+// Returns p1 (== p0: even one tree does not fit).  whole: a budget is taken only when ALL trees [p0, n_trees) fit it
+// (p1 < n_trees on return: the forest does not fit one chunk).
 int forest_chunk(const int32_t* order, int p0, int n_trees, const int32_t* offsets, const int32_t* feature,
                  std::vector<int32_t>& local, std::vector<int32_t>& used, size_t& nodes,
-                 size_t (*bytes)(size_t T, size_t C, size_t Nn)) {
+                 size_t (*bytes)(size_t T, size_t C, size_t Nn), bool whole = false) {
   int p1 = p0;
   for (const size_t budget : {(size_t)kForestSmemBudget, (size_t)(100 * 1024), (size_t)(216 * 1024)}) {
     for (int32_t c : used) local[c] = -1;
@@ -2766,7 +2767,7 @@ int forest_chunk(const int32_t* order, int p0, int n_trees, const int32_t* offse
       used.insert(used.end(), added.begin(), added.end());
       nodes = Nn;
     }
-    if (p1 > p0) break;
+    if (whole ? p1 == n_trees : p1 > p0) break;
   }
   return p1;
 }
@@ -2809,6 +2810,10 @@ size_t forest_predict_bytes(size_t T, size_t C, size_t Nn) {
 size_t forest_classify_bytes(size_t T, size_t C, size_t Nn) {
   return pad_to(8 * T + 8 * T + 8 * C + 8 * Nn + 4 * (T + 1) + 4 * T + 4 * (T + 1), 16) + pad_to(C * kForestTile, 16) +
          T * kForestTile * sizeof(uint16_t);
+}
+// se_forest_weighted_median's shared memory: se_forest_predict's blob and ranks, then the parked keys (uint32)
+size_t forest_wmedian_bytes(size_t T, size_t C, size_t Nn) {
+  return pad_to(forest_predict_bytes(T, C, Nn), 16) + T * kForestTile * sizeof(uint32_t);
 }
 }  // namespace
 
@@ -3020,6 +3025,93 @@ int se_forest_classify(se_ctx* ctx, int which, int kind, int num_classes, int di
                                                   ctx->slot[SE_SLOT_PROB].d, ctx->slot[SE_SLOT_LABEL].d, ctx->sms,
                                                   ctx->stream));
   ctx->last_forest_chunks = chunks;
+  ctx->last_tree_binned = 1;
+  return end(ctx);
+}
+
+// AdaBoost.R2's weighted median of tree members (BoostingRegressionModel.predict, regression/BoostingRegressor.scala:
+// 333-337; ensemble/Utils.scala:26-40) in one pass over the rank matrix: the value se_agg_run selects from the members'
+// outputs, with the same mode choice and the same per-row code, without the [M][n] member outputs.
+int se_forest_weighted_median(se_ctx* ctx, int which, int n_trees, const int32_t* offsets, const int32_t* feature,
+                              const float* threshold, const int32_t* left, const int32_t* right, const float* value,
+                              const double* weights, int out_slot, int out_row) {
+  if (!ctx || !offsets || !feature || !threshold || !left || !right || !value) return fail(ctx, SE_ERR_ARG, "null argument");
+  SE_REQUIRE(ctx, weights, SE_ERR_ARG, "weights required for the weighted median");
+  SE_REQUIRE(ctx, out_slot >= 0 && out_slot < SE_NUM_SLOTS, SE_ERR_ARG, "bad out slot");
+  const SlotBuf& X = ctx->slot[which ? SE_SLOT_VX : SE_SLOT_X];
+  const SlotBuf& O = ctx->slot[out_slot];
+  SE_REQUIRE(ctx, X.d, SE_ERR_STATE, "feature matrix slot not allocated");
+  SE_REQUIRE(ctx, O.d && O.cols == X.cols && out_row >= 0 && out_row < O.rows, SE_ERR_STATE, "output slot shape mismatch");
+  SE_TRY(forest_validate(ctx, X, n_trees, offsets, feature, left, right));
+  SE_REQUIRE(ctx, n_trees <= 64, SE_ERR_STATE,
+             "%d trees: the one-pass weighted median takes at most 64 (evaluate the members with se_tree_predict + se_agg_run)",
+             n_trees);
+  // the whole forest must fit ONE chunk: a row's median needs every member's leaf at once
+  std::vector<int32_t> local((size_t)X.rows, -1);  // global column -> local column
+  std::vector<int32_t> used;
+  size_t nodes = 0;
+  const int t1 = forest_chunk(nullptr, 0, n_trees, offsets, feature, local, used, nodes, forest_wmedian_bytes, true);
+  SE_REQUIRE(ctx, t1 == n_trees, SE_ERR_STATE,
+             "the forest (%d trees, %lld nodes) does not fit one chunk of the weighted-median kernel's shared memory "
+             "(evaluate the members with se_tree_predict + se_agg_run)", n_trees, (long long)offsets[n_trees]);
+  const int64_t total = offsets[n_trees];
+  // mode as se_agg_run picks it: every weight finite and >= 0 -> fast path, all equal -> no rounding margin
+  int mode = 0;
+  if (ctx->wm_fast && X.cols > 0) {
+    bool ok = true, equal = true;
+    for (int i = 0; i < n_trees; ++i) {
+      ok = ok && (weights[i] >= 0.0) && (weights[i] <= 1.7976931348623157e308);
+      equal = equal && (weights[i] == weights[0]);
+    }
+    if (ok) mode = equal ? 2 : 1;
+  }
+  SE_TRY(begin(ctx));
+  release_l2_persist(ctx);
+  SE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  SE_TRY(forest_ranks(ctx, which, X, total, feature, threshold));
+  BinState& B = ctx->bins[which];
+  if (mode == 1 && !ctx->d_wm) {  // the deferred-row count lives where se_agg_run keeps it (d_wm[0])
+    if (cudaMalloc(&ctx->d_wm, sizeof(unsigned int)) == cudaSuccess) ctx->wm_alloc = 1;
+    else { cudaGetLastError(); ctx->d_wm = nullptr; mode = 0; }
+  }
+  if (out_slot == SE_SLOT_F || out_slot == SE_SLOT_R || out_slot == SE_SLOT_Y) ctx->gbm.r_current = false;
+  const size_t T = (size_t)n_trees, C = used.size(), Nn = nodes;
+  ForestWmArgs a;
+  a.X8 = B.d8; a.n = X.cols; a.ld8 = B.ld8;
+  a.out = O.d + (int64_t)out_row * (O.rows > 1 ? O.ld : O.cols);
+  a.T = (int)T; a.C = (int)C;
+  a.off_coloff = (int)(8 * T);
+  a.off_nodes = a.off_coloff + (int)(8 * C);
+  a.off_treeoff = a.off_nodes + (int)(8 * Nn);
+  a.off_values = a.off_treeoff + (int)pad_to(4 * (T + 1), 8);
+  a.blob_bytes = (int)pad_to((size_t)a.off_values + 4 * Nn, 16);
+  a.off_ranks = a.blob_bytes;
+  a.off_parked = a.off_ranks + (int)pad_to(C * kForestTile, 16);
+  std::vector<unsigned char> blob((size_t)a.blob_bytes, 0);
+  double* bw = reinterpret_cast<double*>(blob.data());
+  unsigned long long* bco = reinterpret_cast<unsigned long long*>(blob.data() + a.off_coloff);
+  uint2* bn = reinterpret_cast<uint2*>(blob.data() + a.off_nodes);
+  int32_t* bto = reinterpret_cast<int32_t*>(blob.data() + a.off_treeoff);
+  float* bv = reinterpret_cast<float*>(blob.data() + a.off_values);
+  for (size_t c = 0; c < C; ++c) bco[c] = (unsigned long long)used[c] * (unsigned long long)B.ld8;
+  size_t at = 0;
+  for (int t = 0; t < n_trees; ++t) {
+    const int32_t b = offsets[t], nn = offsets[t + 1] - offsets[t];
+    bw[t] = weights[t];  // fp64, as se_agg_run ships them for the median
+    bto[t] = (int32_t)at;
+    forest_pack_tree(B, local, b, nn, feature, threshold, left, right, bn + at);
+    for (int i = 0; i < nn; ++i) bv[at + i] = value[b + i];
+    at += (size_t)nn;
+  }
+  bto[T] = (int32_t)at;
+  SE_TRY(forest_upload_blob(ctx, blob));
+  a.blob = ctx->d_forest;
+  a.wm_mode = mode;
+  a.weights_host = weights;
+  a.deferred = mode == 1 ? ctx->d_wm : nullptr;
+  SE_LAUNCH_T(ctx, SE_KF_TREE, launch_forest_wmedian(a, ctx->sms, ctx->stream));
+  ctx->last_wm_mode = mode;
+  ctx->last_forest_chunks = 1;
   ctx->last_tree_binned = 1;
   return end(ctx);
 }

@@ -295,6 +295,27 @@ struct ForestClassArgs {
   int64_t ld_raw = 0;
 };
 cudaError_t launch_forest_classify(const ForestClassArgs& a, int sms, cudaStream_t s);
+// The weighted median of a forest's members in ONE pass over the uint8 rank matrix (BoostingRegressionModel.predict
+// with votingStrategy "median", regression/BoostingRegressor.scala:333-337): out[row] = the value se_agg_run
+// (SE_AGG_BOOSTING_REG_MEDIAN) selects from the members' outputs, for T <= 64 trees that fit ONE chunk.  `blob` is
+// ForestArgs' layout (w[T] are the fp64 weights, leaf value per node at off_values) followed in shared memory by
+//   [off_ranks)    uint8    the tile's ranks, [C][256]
+//   [off_parked)   uint32   the leaf value's order-preserving key (wm_key) per tree and row, [T][256]
+// wm_mode 0: exact pick for every row; 1: keys-only sort + model-order bisection, rows inside the margin tau take the
+// exact pick in the same thread and are counted in *deferred; 2: equal weights, fast path for every row.
+struct ForestWmArgs {
+  const uint8_t* X8 = nullptr;
+  int64_t n = 0, ld8 = 0;
+  const unsigned char* blob = nullptr;
+  int blob_bytes = 0;  // multiple of 16
+  int T = 0, C = 0;
+  int off_coloff = 0, off_nodes = 0, off_treeoff = 0, off_values = 0, off_ranks = 0, off_parked = 0;
+  int wm_mode = 0;
+  const double* weights_host = nullptr;  // [T], host memory: the fast path's constant-bank operands
+  unsigned int* deferred = nullptr;      // mode 1: rows that took the exact pick (zeroed by the launcher)
+  float* out = nullptr;
+};
+cudaError_t launch_forest_wmedian(const ForestWmArgs& a, int sms, cudaStream_t s);
 // The classifier aggregations' epilogue (se_agg.cu agg_finalize_kernel) over the stage-1 sums already in raw[C][ld]:
 // raw, prob and label as se_agg_run writes them.  M: members (bagging: prob = raw / M); sum_a: Σ a_m (SAMME).
 cudaError_t launch_agg_finalize(int kind, int C, int K, int dim, int loss, int M, double sum_a, int64_t n, int64_t ld,

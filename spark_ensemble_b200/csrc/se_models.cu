@@ -9,6 +9,7 @@
 #include <stdlib.h>
 
 #include "se_kernels.h"
+#include "se_wmedian.cuh"
 
 namespace se {
 
@@ -482,6 +483,133 @@ __global__ void __launch_bounds__(kForestTile, 2) forest_classify_kernel(const F
   }
 }
 
+// The same tile for the weighted median of the members (AdaBoost.R2, votingStrategy "median").  The median needs all
+// T leaf values of a row at once, so phase 1 parks each tree's leaf as its order-preserving 32-bit key (wm_key) in the
+// thread's own column of shared memory, [T][256], and phase 2 selects from them in registers with the aggregation's
+// own per-row code (se_wmedian.cuh): the keys-only sort and model-order bisection of the fast path, and the exact
+// (key, model) pick for mode 0 and for the rows whose decision lies inside the rounding margin.  The exact pick runs
+// in the same thread from the parked keys, so no row list and no second pass over the ranks exist; it reloads the
+// keys rather than keeping them, so the fast path's keys and the exact pick's words are never live together.  At
+// MP = 64 the bisection reads the model-order keys from the parked column in a rolled loop instead of a second
+// register copy: with both 64-key copies in registers (agg_wmedian_fast_kernel: 246) this kernel spilled; so it uses
+// 207 registers and no local memory.
+template <int MP>
+__global__ void __launch_bounds__(kForestTile, (MP >= 32) ? 1 : 2)
+    forest_wmedian_kernel(const ForestWmArgs a, const __grid_constant__ WmWeights wts, const double total, const double tau) {
+  extern __shared__ __align__(16) unsigned char fsm[];
+  for (int i = threadIdx.x; i < a.blob_bytes / 16; i += kForestTile)
+    reinterpret_cast<uint4*>(fsm)[i] = __ldg(reinterpret_cast<const uint4*>(a.blob) + i);
+  const double* s_w = reinterpret_cast<const double*>(fsm);
+  const unsigned long long* s_coloff = reinterpret_cast<const unsigned long long*>(fsm + a.off_coloff);
+  const uint2* s_nodes = reinterpret_cast<const uint2*>(fsm + a.off_nodes);
+  const int* s_toff = reinterpret_cast<const int*>(fsm + a.off_treeoff);
+  const float* s_val = reinterpret_cast<const float*>(fsm + a.off_values);
+  unsigned char* s_rank = fsm + a.off_ranks;
+  uint32_t* s_park = reinterpret_cast<uint32_t*>(fsm + a.off_parked) + threadIdx.x;  // this thread's column
+  const int M = a.T;
+  const double half = 0.5 * total;
+  constexpr int LOG = (MP == 1) ? 0 : (MP == 2) ? 1 : (MP == 4) ? 2 : (MP == 8) ? 3 : (MP == 16) ? 4 : (MP == 32) ? 5 : 6;
+  const int64_t ntiles = (a.n + kForestTile - 1) / kForestTile;
+  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    __syncthreads();  // the packed trees are staged (first tile) / the previous tile's ranks are no longer read
+    const int64_t row0 = tile * kForestTile;
+    for (int i = threadIdx.x; i < a.C * (kForestTile / 4); i += kForestTile) {
+      const int c = i / (kForestTile / 4), q = i % (kForestTile / 4);
+      const int64_t r = row0 + 4 * q;  // columns are padded to 128 rows: a word at r < ld8 stays inside its column
+      uint32_t v = 0;
+      if (r < a.ld8) v = __ldg(reinterpret_cast<const uint32_t*>(a.X8 + s_coloff[c] + r));
+      *reinterpret_cast<uint32_t*>(s_rank + c * kForestTile + 4 * q) = v;
+    }
+    __syncthreads();
+    const int64_t row = row0 + threadIdx.x;
+    if (row >= a.n) continue;  // no barrier or warp collective below: a thread only reads back what it parked itself
+    const unsigned char* myr = s_rank + threadIdx.x;
+    int t = 0;
+    for (; t + 1 < M; t += 2) {  // two independent walks in flight
+      const uint2* n0 = s_nodes + s_toff[t];
+      const uint2* n1 = s_nodes + s_toff[t + 1];
+      int d0 = 0, d1 = 0;
+      bool l0 = true, l1 = true;
+      while (l0 || l1) {
+        if (l0) forest_step(n0, myr, d0, l0);
+        if (l1) forest_step(n1, myr, d1, l1);
+      }
+      s_park[t * kForestTile] = wm_key(s_val[s_toff[t] + d0]);
+      s_park[(t + 1) * kForestTile] = wm_key(s_val[s_toff[t + 1] + d1]);
+    }
+    if (t < M) {
+      int d0 = 0;
+      bool l0 = true;
+      while (l0) forest_step(s_nodes + s_toff[t], myr, d0, l0);
+      s_park[t * kForestTile] = wm_key(s_val[s_toff[t] + d0]);
+    }
+    auto leaf_key = [&](int m) { return s_park[m * kForestTile]; };
+    constexpr bool kRegKeys = MP < 64;  // model-order keys in registers, or read back from the parked column
+    bool exact = a.wm_mode == 0;
+    uint32_t v_hi = 0;
+    if (!exact) {  // the fast path of agg_wmedian_fast_kernel, row for row
+      uint32_t key[kRegKeys ? MP : 1], s[MP];
+#pragma unroll
+      for (int m = 0; m < MP; ++m) {
+        s[m] = 0xFFFFFFFFu;  // padding sorts last and carries weight 0
+        if (m < M) s[m] = leaf_key(m);
+        if constexpr (kRegKeys) key[m] = s[m];
+      }
+      sortnet_oddeven<MP>(s, [](uint32_t& x, uint32_t& y) {
+        const uint32_t lo = min(x, y), hi = max(x, y);
+        x = lo;
+        y = hi;
+      });
+      // invariant: P(lo) false, P(hi) true with P(k) := Ĉ(s[k]) >= ĥ; lo = t - 1, hi = t after LOG probes
+      uint32_t tt = 0;
+      v_hi = s[MP - 1];
+      double c_lo = 0.0, c_hi = total;
+      auto probe = [&](uint32_t v) {
+        double c = 0.0;
+        if constexpr (kRegKeys) {
+#pragma unroll
+          for (int m = 0; m < MP; ++m) {
+            const double b = __hiloint2double((key[m] <= v) ? 0x3ff00000 : 0, 0);
+            c = fma(wts.w[m], b, c);
+          }
+        } else {  // a rolled loop over the parked column: weights by index from the parameter bank (m >= M: weight 0)
+#pragma unroll 4
+          for (int m = 0; m < M; ++m) {
+            const double b = __hiloint2double((leaf_key(m) <= v) ? 0x3ff00000 : 0, 0);
+            c = fma(wts.w[m], b, c);
+          }
+        }
+        const bool right = !(c >= half);
+        c_lo = right ? c : c_lo;
+        c_hi = right ? c_hi : c;
+        v_hi = right ? v_hi : v;
+        tt = 2u * tt + (right ? 1u : 0u);
+      };
+      if constexpr (LOG > 0) probe(wm_candidate<MP, 0>(s, tt));
+      if constexpr (LOG > 1) probe(wm_candidate<MP, 1>(s, tt));
+      if constexpr (LOG > 2) probe(wm_candidate<MP, 2>(s, tt));
+      if constexpr (LOG > 3) probe(wm_candidate<MP, 3>(s, tt));
+      if constexpr (LOG > 4) probe(wm_candidate<MP, 4>(s, tt));
+      if constexpr (LOG > 5) probe(wm_candidate<MP, 5>(s, tt));
+      const bool safe = (c_hi - half > tau) && (half - c_lo > tau);
+      if (a.wm_mode == 1 && !safe) {  // the decision could depend on the order of summation
+        exact = true;
+        atomicAdd(a.deferred, 1u);
+      }
+    }
+    if (exact) {
+      unsigned long long w[MP];
+#pragma unroll
+      for (int m = 0; m < MP; ++m) {
+        w[m] = ~0ull;  // padding sorts last
+        if (m < M) w[m] = ((unsigned long long)leaf_key(m) << 32) | (unsigned long long)(unsigned)m;
+      }
+      v_hi = (uint32_t)(wm_exact_pick<MP>(w, M, s_w) >> 32);
+    }
+    a.out[row] = wm_unkey(v_hi);
+  }
+}
+
 constexpr int LU = 8;
 
 __global__ void __launch_bounds__(kBlock) linear_predict_kernel(const float* __restrict__ X, int64_t n,
@@ -632,6 +760,52 @@ cudaError_t launch_forest_classify(const ForestClassArgs& a, int sms, cudaStream
   if (need < 1) need = 1;
   const int64_t cap = (int64_t)sms * per_sm;
   kern<<<(int)(need < cap ? need : cap), kForestTile, smem, st>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_forest_wmedian(const ForestWmArgs& a, int sms, cudaStream_t st) {
+  const size_t smem = (size_t)a.off_parked + (size_t)a.T * kForestTile * sizeof(uint32_t);
+  if (a.T < 1 || a.T > 64 || a.C < 0 || smem > 220 * 1024 || (a.blob_bytes & 15) != 0 || (a.off_parked & 15) != 0 ||
+      (a.wm_mode != 0 && a.weights_host == nullptr) || (a.wm_mode == 1 && a.deferred == nullptr))
+    return cudaErrorInvalidValue;
+  WmWeights wts;
+  double total = 0.0, tau = -1.0;
+  if (a.wm_mode != 0) {
+    wm_fast_operands(a.weights_host, a.T, a.wm_mode, &wts, &total, &tau);
+  } else {
+    for (int m = 0; m < 64; ++m) wts.w[m] = 0.0;  // unused: the exact pick reads the blob's weights
+  }
+  if (a.wm_mode == 1) {
+    const cudaError_t e = cudaMemsetAsync(a.deferred, 0, sizeof(unsigned int), st);
+    if (e != cudaSuccess) return e;
+  }
+  int Mp = 1;
+  while (Mp < a.T) Mp <<= 1;
+  void (*kern)(const ForestWmArgs, const WmWeights, const double, const double) = nullptr;
+  switch (Mp) {
+    case 1: kern = forest_wmedian_kernel<1>; break;
+    case 2: kern = forest_wmedian_kernel<2>; break;
+    case 4: kern = forest_wmedian_kernel<4>; break;
+    case 8: kern = forest_wmedian_kernel<8>; break;
+    case 16: kern = forest_wmedian_kernel<16>; break;
+    case 32: kern = forest_wmedian_kernel<32>; break;
+    default: kern = forest_wmedian_kernel<64>; break;
+  }
+  if (smem > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  // resident CTAs per SM from registers and shared memory together
+  int per_sm = 1;
+  {
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kForestTile, smem);
+    if (e != cudaSuccess) return e;
+  }
+  if (per_sm < 1) per_sm = 1;
+  int64_t need = (a.n + kForestTile - 1) / kForestTile;
+  if (need < 1) need = 1;
+  const int64_t cap = (int64_t)sms * per_sm;
+  kern<<<(int)(need < cap ? need : cap), kForestTile, smem, st>>>(a, wts, total, tau);
   return cudaGetLastError();
 }
 

@@ -60,8 +60,8 @@ def _split_validation(est: Params, dataset: DataFrame):
 
 
 # Param `forestTransform` of the tree-ensemble models: transform evaluates the whole forest in one pass over the
-# feature matrix on the device (se_forest_predict / se_forest_classify) instead of predicting every member on the host
-# and aggregating the stacked outputs.  Off by default.
+# feature matrix on the device (se_forest_predict / se_forest_classify / se_forest_weighted_median) instead of
+# predicting every member on the host and aggregating the stacked outputs.  Off by default.
 _pforest = [Param("forestTransform", "transform tree ensembles in one pass over the device-resident features", convert=bool)]
 
 
@@ -378,6 +378,10 @@ class BoostingRegressor(Params):
         ctx = Context(self.device)
         try:
             ctx.boostreg_configure(n)
+            resident = bool(self("residentFeatures"))
+            if resident:  # column-major X in HBM: fitted trees / linear models are evaluated on device (no upload per round)
+                ctx.alloc(N.SLOT_X, X.shape[1], n)
+                ctx.upload_rowmajor(N.SLOT_X, X)
             ctx.upload(N.SLOT_Y, y)
             ctx.upload(N.SLOT_BW, np.ones(n) if w is None else w)  # :205
             sum_w = ctx.slot_sum(N.SLOT_BW)                          # :212
@@ -385,7 +389,7 @@ class BoostingRegressor(Params):
             while i < self("numBaseLearners") and not done and sum_w > 0:  # :218
                 wn = ctx.download(N.SLOT_BW, scale=1.0 / sum_w)     # :222-225
                 model = learner.fit(X, y, wn)                        # third party :231-233
-                ctx.upload(N.SLOT_PRED, model.predict(X))
+                _predict_into(ctx, model, X, resident)
                 max_error = ctx.boostreg_max_error()                 # :235-238
                 if max_error == 0:                                   # :240-243
                     best, done = i, True
@@ -410,14 +414,36 @@ class BoostingRegressor(Params):
             ctx.close()
 
 
+def _predict_into(ctx: Context, model, X, resident: bool):
+    """The member's predictions in SLOT_PRED: on the device over the resident X for a tree or a linear model, otherwise
+    model.predict on the host + upload (the reference's path)."""
+    t = model.tree_arrays() if resident else None
+    if t is not None:
+        ctx.tree_predict(t, N.SLOT_PRED, 0)
+        return
+    lin = model.linear_arrays() if resident else None
+    if lin is not None:
+        ctx.linear_predict(lin["coef"], float(lin["intercept"]), N.SLOT_PRED, 0)
+        return
+    ctx.upload(N.SLOT_PRED, model.predict(X))
+
+
+def _forest_median(ctx: Context, trees, weights) -> np.ndarray:
+    n = ctx.layout(N.SLOT_X)[1]
+    ctx.alloc(N.SLOT_RAW, 1, n)
+    ctx.forest_weighted_median(trees, N.SLOT_RAW, weights)
+    return ctx.download(N.SLOT_RAW).astype(np.float64)
+
+
 _pbr = [Param("lossType", "loss function, exponential by default (case-insensitive). Supported: exponential,squared,linear",
               lambda v: v.lower() in ("exponential", "squared", "linear"), str),
         Param("votingStrategy", "voting strategy, (case-insensitive). Supported options: median,mean",
               lambda v: v.lower() in ("median", "mean"), str),
-        Param("seed", "random seed", convert=int)]
-_BOOST_REG_DEFAULTS = {**_d, **_db, "lossType": "exponential", "votingStrategy": "median",
-                       "seed": java_string_hash("org.apache.spark.ml.regression.BoostingRegressor")}
-BoostingRegressor._declare(_p + _pb + _pbr, _BOOST_REG_DEFAULTS)
+        Param("seed", "random seed", convert=int),
+        Param("residentFeatures", "evaluate base models on device over the HBM-resident feature matrix", convert=bool)]
+_BOOST_REG_DEFAULTS = {**_d, **_db, "lossType": "exponential", "votingStrategy": "median", "residentFeatures": False,
+                       "forestTransform": False, "seed": java_string_hash("org.apache.spark.ml.regression.BoostingRegressor")}
+BoostingRegressor._declare(_p + _pb + _pbr + _pforest, _BOOST_REG_DEFAULTS)
 
 
 class BoostingRegressionModel(Params):
@@ -433,8 +459,22 @@ class BoostingRegressionModel(Params):
         self.parent = None
 
     def _aggregate(self, X) -> np.ndarray:
+        median = self("votingStrategy").lower() == "median"
+        trees = _member_trees(self.models) if self("forestTransform") else None
+        if trees is not None:
+            if median:  # the weighted median of the leaves, fused with the forest walk (se_forest_weighted_median)
+                run = lambda ctx: _forest_median(ctx, trees, self.weights)
+            else:  # dot(predictions, weights) / Σ weights (BoostingRegressor.scala:339-342) as Σ_i (w_i / Σw) · m_i
+                sum_w = 0.0
+                for a in self.weights:  # fp64, model order
+                    sum_w += float(a)
+                run = lambda ctx: _forest_predict(ctx, trees, None, self.weights / sum_w, 0.0)
+            # None: more than 64 members, a forest beyond one chunk or a column with > 255 thresholds (member route)
+            out = _forest_transform(self.device, X, run)
+            if out is not None:
+                return out
         P = np.ascontiguousarray(np.stack([m.predict(X) for m in self.models]), dtype=np.float32)
-        kind = N.AGG_BOOSTING_REG_MEDIAN if self("votingStrategy").lower() == "median" else N.AGG_BOOSTING_REG_MEAN
+        kind = N.AGG_BOOSTING_REG_MEDIAN if median else N.AGG_BOOSTING_REG_MEAN
         with Context(self.device) as ctx:
             ctx.agg_configure(kind, P.shape[0], 0, 1, 0, X.shape[0])
             ctx.upload(N.SLOT_P, P)
@@ -448,4 +488,4 @@ class BoostingRegressionModel(Params):
         return float(self._aggregate(np.asarray(features).reshape(1, -1))[0])
 
 
-BoostingRegressionModel._declare(_p + _pb + _pbr, _BOOST_REG_DEFAULTS)
+BoostingRegressionModel._declare(_p + _pb + _pbr + _pforest, _BOOST_REG_DEFAULTS)

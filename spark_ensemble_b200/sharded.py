@@ -225,6 +225,10 @@ class ShardedContext:
         self._all(lambda r, c: c.forest_classify(trees, kind, num_classes, dim=dim, loss=loss, weights=weights, init=init,
                                                  validation=validation, subspaces=subspaces))
 
+    def forest_weighted_median(self, trees, out_slot, weights, out_row=0, validation=False):
+        """Every shard takes the weighted median over its own rows (no reduction)."""
+        self._all(lambda r, c: c.forest_weighted_median(trees, out_slot, weights, out_row=out_row, validation=validation))
+
     def linear_predict(self, coef, intercept, out_slot, out_row=0, validation=False, subspace=None):
         self._all(lambda r, c: c.linear_predict(coef, intercept, out_slot, out_row, validation=validation, subspace=subspace))
 
